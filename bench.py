@@ -3,6 +3,10 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched under torchrun)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR
+
+--dump-outputs writes what the timed path computed in its last step as DIR/<name>.npy (float32, or float64 where
+float32 would round), so that two builds can be compared output for output on the same seeded inputs.
 
 A "step" is one pass of the hot path over one batch: forward + reverse fill with packed
 traceback and the near-optimal cell set for the C3 workload (100k synthetic protein pairs,
@@ -109,6 +113,61 @@ def load_peaks():
         d = json.load(open(p))
         return float(d["hbm_gbs"]), "measured (MEASURED_PEAKS.json)", float(d.get("sm_max_mhz", 1965.0))
     return 6650.0, "fallback (B200_PROFILING.md)", 1965.0
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, rank, arrays):
+    """Write each array as <dirname>/<name>.npy (rank > 0: <name>.rank<r>.npy).  Integers become float32 when every
+    value is exact in float32, float64 otherwise."""
+    conv = {}
+    for name, arr in arrays.items():
+        arr = np.asarray(arr)
+        if arr.dtype == np.float32 or arr.dtype == np.uint8:
+            arr = arr.astype(np.float32)
+        elif arr.dtype.kind in "iu" and (arr.size == 0 or int(np.abs(arr).max()) < (1 << 24)):
+            arr = arr.astype(np.float32)
+        else:
+            arr = arr.astype(np.float64)
+        conv[name] = arr
+    total = sum(a.nbytes for a in conv.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes, more than the %d allowed" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(dirname, exist_ok=True)
+    suffix = "" if rank == 0 else ".rank%d" % rank
+    for name, arr in conv.items():
+        np.save(os.path.join(dirname, name + suffix + ".npy"), arr)
+
+
+def batch_outputs(ctx, a, what, d_f, d_r, d_t, d_c, seqs=None, pq=None, pt=None, sample_pairs=0):
+    """What a caller of aadp_run_batch receives: the per-pair arrays it asked for and, for a fixed seeded sample of
+    pairs, the resident matrices it can fetch with aadp_batch_fetch_pair (flattened and concatenated in sample order)."""
+    out = {}
+    if what & a.W_FWD:
+        out["fwd_score"] = d_f.cpu().numpy()
+    if what & a.W_REV:
+        out["rev_score"] = d_r.cpu().numpy()
+    if what & a.W_MASK:
+        out["threshold"] = d_t.cpu().numpy()
+        out["nearopt_count"] = d_c.cpu().numpy()
+    if sample_pairs and (what & a.W_TB):
+        n = len(pq)
+        ids = np.sort(np.random.default_rng(0).choice(n, min(sample_pairs, n), replace=False))
+        parts = {}
+        for p in ids:
+            Lq, Lt = len(seqs[pq[p]]), len(seqs[pt[p]])
+            # without W_SCORES the reverse score matrix is never materialised: reverse traceback only
+            got = ctx.fetch_pair(int(p), Lq, Lt, fwd=True, rev=False, mask=bool(what & a.W_MASK))
+            got.update({k: v for k, v in ctx.fetch_pair(int(p), Lq, Lt, fwd=False, rev=True, scores=False).items()
+                        if v is not None})
+            for k, v in got.items():
+                if v is not None:
+                    parts.setdefault(k, []).append(v.ravel())
+        out["sample_pair_ids"] = ids
+        for k, v in parts.items():
+            out["sample_" + k] = np.concatenate(v)
+    return out
 
 
 def make_workload(rank, npairs):
@@ -281,6 +340,12 @@ def run_c4(args, rank, local_rank, world, barrier, max_over_ranks, sum_over_rank
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     prof = ctx.profile()
     ctx.set_profiling(False)
+    if emit and args.dump_outputs:
+        # the score blocks of this rank's rectangles, concatenated: a fixed seeded sample of them
+        n_sc = d_scores.numel()
+        idx = np.unique(np.random.default_rng(0).integers(0, n_sc, 1 << 20)) if n_sc else np.zeros(0, np.int64)
+        dump_outputs(args.dump_outputs, rank, {
+            "scores_sample": d_scores[torch.from_numpy(idx).cuda()].cpu().numpy(), "scores_sample_index": idx})
     value = useful_cu * args.steps / (ms_total * 1e-3) / 1e9
     # ---- end to end: sequences from pinned host memory, every score block back to the host
     def step_e2e():
@@ -343,7 +408,8 @@ def run_c4(args, rank, local_rank, world, barrier, max_over_ranks, sum_over_rank
     return line
 
 
-def quick_pairlist(workload, args, rank, local_rank, world, barrier, max_over_ranks, sum_over_ranks, steps, warmup):
+def quick_pairlist(workload, args, rank, local_rank, world, barrier, max_over_ranks, sum_over_ranks, steps, warmup,
+                   dump_dir=None):
     """Device-timed value of one of the pair-list workloads (inputs resident), for the `extra` keys of the default
     line: c2 (10k pairs forward score-only) and c5 (one 30k x 30k pair fwd+rev+traceback+mask, one replica per rank)."""
     import torch
@@ -391,6 +457,8 @@ def quick_pairlist(workload, args, rank, local_rank, world, barrier, max_over_ra
     ms = max_over_ranks(e0.elapsed_time(e1))
     prof = ctx.profile()
     ctx.set_profiling(False)
+    if dump_dir:
+        dump_outputs(dump_dir, rank, batch_outputs(ctx, a, what, d_f, d_r, d_t, d_c))
     if (what & a.W_REV) and workload != "c3f":  # (fp32 scoring: the two directions round differently)
         assert torch.equal(d_f, d_r), "forward and reverse optima differ"
     by = {}
@@ -460,7 +528,14 @@ def main():
     ap.add_argument("--long-len", type=int, default=30000)
     ap.add_argument("--no-extras", action="store_true",
                     help="default (c3) run only: skip the `extra` keys (C2, C4 strong scaling, C5, alignments end to end)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last step as DIR/<name>.npy (at most 64 MB; "
+                         "larger outputs as a fixed seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs the GPU implementation")
     rank, local_rank, world = env_int("RANK", 0), env_int("LOCAL_RANK", 0), env_int("WORLD_SIZE", 1)
     if args.impl == "reference":
         run_reference_arm(args, rank, world)
@@ -505,7 +580,8 @@ def main():
             dist.destroy_process_group()
         return
     if args.workload == "c3f":  # the C3 shape under the reference's default (non-dyadic) penalties: exact fp32 path
-        r = quick_pairlist("c3f", args, rank, local_rank, world, barrier, max_over_ranks, sum_over_ranks, max(1, args.steps // 5), 1)
+        r = quick_pairlist("c3f", args, rank, local_rank, world, barrier, max_over_ranks, sum_over_ranks, args.steps, 1,
+                           args.dump_outputs)
         if rank == 0:
             print(json.dumps({"metric": "GCUPS fwd+rev exact fp32 general-gap fill + near-optimal counts", "n_gpus": world,
                               "higher_is_better": True, "data": "synthetic", "vs_baseline": None, **r}), flush=True)
@@ -584,6 +660,9 @@ def main():
     total_cu = sum_over_ranks(cu_step)
     value = total_cu * args.steps / (ms_total * 1e-3) / 1e9
     ms_per_step = ms_total / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, rank, batch_outputs(ctx, a, what, d_f, d_r, d_t, d_c, seqs, pq, pt,
+                                                           8 if args.workload == "c3" else 0))
 
     # correctness guard inside the bench: the two directions must agree on every optimum
     if what & a.W_REV:
@@ -617,7 +696,7 @@ def main():
         pairs_t = torch.empty((cap_rows, 2), dtype=torch.int32).pin_memory()
         n_t = torch.empty(n, dtype=torch.int32).pin_memory()
         st_t = torch.empty(n, dtype=torch.int32).pin_memory()
-        asteps = max(2, min(args.steps, 5))
+        asteps = args.steps
 
         def step_ali():
             ctx.fill_batch(hb["res"], hb["off"], hb["pq"], hb["pt"], what, DELTA)

@@ -1,17 +1,17 @@
 """The C++ drop-in boundary: one demo source (tests/cxx/dropin_demo.cpp, shaped like the reference
 driver aa_ali.cpp:63-90) is compiled against this repo's include/hmap2 headers (GPU fill) and against
-the unmodified reference headers (CPU).  Their DPCell dumps and optimal alignments must be identical."""
+the unmodified reference headers (CPU).  Their DPCell dumps and optimal alignments must be identical.
+The reference builds' output is stored in tests/golden/reference_digests.json (tests/util.py, ReferenceResults)."""
 import os
 import subprocess
 
 import numpy as np
 import pytest
 
-from util import ROOT, po, MODES, MODE_NAMES
+from util import ROOT, po, MODES, MODE_NAMES, ReferenceResults
 
 CXX = os.path.join(ROOT, "tests", "cxx")
 DEMO = os.path.join(CXX, "dropin_demo")
-REF_DEMO = os.path.join(CXX, "ref_demo")
 MATRIX = os.path.join(ROOT, "alignment_algos_b200", "data", "BLOSUM62")
 ALPHA = "ARNDCQEGHILKMFPSTWYVBZX*"
 
@@ -44,23 +44,23 @@ def _expected_lines(O, q, t, sub, fast=True):
 def test_headers_compile_and_reference_demo_matches_oracle(blosum):
     subprocess.check_call(["make", "-C", CXX, "all"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
     assert os.path.exists(DEMO)
-    if not os.path.exists(REF_DEMO):
-        pytest.skip("reference demo not built")
     _, M = blosum
+    ref = ReferenceResults("test_cxx_dropin.py::test_headers_compile_and_reference_demo_matches_oracle")
     rng = np.random.default_rng(21)
     for at in (po.GLOBAL, po.SEMI_LOCAL, po.LOCAL):
         q = rng.integers(0, 20, 23).astype(np.uint8)
         t = rng.integers(0, 20, 31).astype(np.uint8)
         O = po.Oracle(M, 12, 1, at)
         want, _ = _expected_lines(O, q, t, M)
-        got = [l for l in _run(REF_DEMO, at, 12, 1, q, t) if l[:2] in ("F ", "R ")]
-        assert got == want
+        ref.check("DPCell lines of the reference demo, mode %d" % at, want)
+    ref.close()
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("at", MODES, ids=[MODE_NAMES[m] for m in MODES])
 def test_gpu_dropin_equals_reference_build(blosum, at):
     _, M = blosum
+    ref = ReferenceResults("test_cxx_dropin.py::test_gpu_dropin_equals_reference_build[%s]" % MODE_NAMES[at])
     rng = np.random.default_rng(40 + at)
     # the last case is the reference's default scoring (alib.cpp:17-18): not on a dyadic grid -> exact fp32 path
     for (gi, ge, Lq, Lt) in [(12, 1, 37, 52), (3, 1, 64, 20), (10.5, 0.25, 18, 18), (12, 1, 1, 9), (12, 1, 300, 270),
@@ -72,13 +72,12 @@ def test_gpu_dropin_equals_reference_build(blosum, at):
         O = po.Oracle(M, gi, ge, at)
         want, res = _expected_lines(O, q, t, M, fast=(gi != 4.73))
         assert core[:len(want)] == want
-        if os.path.exists(REF_DEMO) and Lq * Lt < 5000:
-            ref_all = _run(REF_DEMO, at, gi, ge, q, t)
-            ref = [l for l in ref_all if not l.startswith("#") and not l.startswith("@")]
-            assert core == ref, "GPU drop-in build and reference build print different results"
+        if Lq * Lt < 5000:
+            case = "%s %s %dx%d" % (gi, ge, Lq, Lt)
+            ref.check("everything the reference build prints, " + case, core)
             # near-optimal alignments (ucw.h) enumerated on the GPU vs. the reference recursion: same set, same scores
-            ucw_got, ucw_ref = sorted(l for l in got if l.startswith("@")), sorted(l for l in ref_all if l.startswith("@"))
-            assert ucw_got == ucw_ref, "GPU enumeration and the reference's UnconstrainedNearOptimal differ"
+            ucw_got = sorted(l for l in got if l.startswith("@"))
+            ref.check("UnconstrainedNearOptimal alignments of the reference build, " + case, ucw_got)
             if at != po.LOCAL:
                 assert len(ucw_got) >= 2
             if Lq > 7 and Lt > 7:  # the loop list closed in ONE aadp_fill_subpair_batch call vs. one sub-matrix per loop
@@ -102,6 +101,7 @@ def test_gpu_dropin_equals_reference_build(blosum, at):
             mask, cnt = O.nearopt_mask(F, R, O.sim(q, t), thr)
             no = [l for l in got if l.startswith("#NEAROPT")][0].split()
             assert int(no[-1]) == cnt and float(no[4]) == pytest.approx(thr, rel=1e-6)
+    ref.close()
 
 
 REFPATCH_GPU = os.path.join(CXX, "refpatch_gpu")
@@ -137,7 +137,6 @@ def test_unmodified_reference_with_gpu_fill_enumerates_the_same_alignments(at):
 
 
 TAB_DEMO = os.path.join(CXX, "tabeval_demo")
-TAB_REF = os.path.join(CXX, "tabeval_ref")
 
 
 @pytest.mark.gpu
@@ -146,8 +145,9 @@ def test_user_evaluator_with_positional_gaps_equals_reference_build(at):
     # tests/cxx/tabeval_demo.cpp: a user-defined Evaluator whose gap penalties depend on the template position
     # (hmap_eval.h:63-117 / gn2_eval.h:99-158 shaped).  hmap2::DPMatrix tabulates it and fills on the GPU
     # (aadp_fill_pair_tabulated); the unmodified reference fills on the CPU.  Same source, identical output.
-    if not (os.path.exists(TAB_DEMO) and os.path.exists(TAB_REF)):
-        pytest.skip("tabeval demos not built")
+    assert os.path.exists(TAB_DEMO), "tests/cxx/tabeval_demo is built by __graft_entry__.build()"
+    ref = ReferenceResults("test_cxx_dropin.py::test_user_evaluator_with_positional_gaps_equals_reference_build[%s]"
+                           % MODE_NAMES[at])
     rng = np.random.default_rng(70 + at)
     for style in (1, 2):
         for (gi, ge, Lq, Lt) in [(4.73, 0.34, 33, 47), (7.1, 0.9, 5, 1), (10, 0.5, 80, 75)]:
@@ -155,15 +155,13 @@ def test_user_evaluator_with_positional_gaps_equals_reference_build(at):
             t = rng.integers(0, 20, Lt).astype(np.uint8)
             args = [MATRIX, str(at), str(gi), str(ge), str(style), _letters(q), _letters(t)]
             got = subprocess.run([TAB_DEMO] + args, capture_output=True, text=True, timeout=120)
-            ref = subprocess.run([TAB_REF] + args, capture_output=True, text=True, timeout=300)
-            assert ref.returncode == 0, ref.stdout[-300:] + ref.stderr[-300:]
             assert got.returncode == 0, got.stdout[-300:] + got.stderr[-300:]
-            assert len(ref.stdout.splitlines()) == 2 * (Lq + 2) * (Lt + 2) + 1
-            assert got.stdout == ref.stdout, "style %d %dx%d: GPU tabulated fill differs from the reference build" % (style, Lq, Lt)
+            assert len(got.stdout.splitlines()) == 2 * (Lq + 2) * (Lt + 2) + 1
+            ref.check("style %d %dx%d: output of the reference build" % (style, Lq, Lt), got.stdout)
+    ref.close()
 
 
 PRUNED_DEMO = os.path.join(CXX, "pruned_demo")
-PRUNED_REF = os.path.join(CXX, "pruned_ref")
 
 
 def _run_pruned(binary, at, gi, ge, delta, kl, sl, mo, flags, q, t):
@@ -180,8 +178,9 @@ def test_pruned_enumerators_dropin_equals_reference_build(at):
     # SURVEY.md §8 row f2: include/hmap2/kscw.h + crcw.h (GPU fill + aadp_batch_near_optimal_pruned) against the UNMODIFIED
     # reference headers compiled from the same source: the printed alignment sets (scores and aligned pairs, after the
     # reference's sortSet) must be the same.  Alignments of equal score may be listed in either order.
-    if not (os.path.exists(PRUNED_DEMO) and os.path.exists(PRUNED_REF)):
-        pytest.skip("pruned demos not built")
+    assert os.path.exists(PRUNED_DEMO), "tests/cxx/pruned_demo is built by __graft_entry__.build()"
+    ref = ReferenceResults("test_cxx_dropin.py::test_pruned_enumerators_dropin_equals_reference_build[%s]"
+                           % MODE_NAMES[at])
     rng = np.random.default_rng(60 + at)
     n = 0
     for gi, ge in ((3, 1), (12, 1), (4.73, 0.34)):
@@ -193,12 +192,12 @@ def test_pruned_enumerators_dropin_equals_reference_build(at):
             for flags in (None, (np.arange(len(t) + 2) // 7) % 2):
                 for kl, sl, mo in ((16, 100, 0.3), (4, 10, 0.5)):
                     got = _run_pruned(PRUNED_DEMO, at, gi, ge, delta, kl, sl, mo, flags, q, t)
-                    ref = _run_pruned(PRUNED_REF, at, gi, ge, delta, kl, sl, mo, flags, q, t)
-                    assert [l for l in got if " n " in l] == [l for l in ref if " n " in l]
-                    assert sorted(got) == sorted(ref), (gi, ge, L, kl)
+                    ref.check("%s %s %d %d: output of the reference build" % (gi, ge, L, kl),
+                              [l for l in got if " n " in l], sorted(got))
                     # sortSet order: scores must be non-increasing in both
                     for tag in ("KS", "CR"):
                         sc = [float(l.split()[1]) for l in got if l.startswith(tag + " ") and " pairs" in l]
                         assert sc == sorted(sc, reverse=True)
                     n += len(got)
+    ref.close()
     assert n > 200

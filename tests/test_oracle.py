@@ -1,9 +1,8 @@
-"""CPU tests: pin the C restatement (oracle/aadp_oracle.c) against the real reference and the
+"""CPU tests: pin the C restatement (oracle/aadp_oracle.c) against the real reference's results and the
 committed golden vectors, and check the domain properties the GPU tests rely on."""
 import numpy as np
-import pytest
 
-from util import po, HAVE_REF, MODES, golden_cases, golden_case, rand_pair, assert_matrix_equal
+from util import po, MODES, ReferenceResults, golden_cases, golden_case, rand_pair, assert_matrix_equal
 
 
 def test_oracle_matches_golden(golden):
@@ -37,34 +36,28 @@ def test_revbug_case_b5(golden):
     assert (pq[0, 0], pt[0, 0]) == (5, 1)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference library not built")
 def test_oracle_matches_reference_random(blosum):
-    alpha, M = blosum
+    _, M = blosum
+    ref = ReferenceResults("test_oracle.py::test_oracle_matches_reference_random")
     rng = np.random.default_rng(7)
     cells = 0
     for gi, ge in [(12, 1), (3, 1), (2, 2), (10.5, 0.25), (1, 0)]:
         for at in MODES:
             O = po.Oracle(M, gi, ge, at)
-            R = po.Reference(alpha, M, gi, ge, at)
             for trial in range(6):
                 Lq, Lt = int(rng.integers(0, 36)), int(rng.integers(0, 36))
                 q, t = rand_pair(rng, Lq, Lt, 24)
                 for d in (po.FWD, po.REV):
-                    rs, rq, rt, rsim = R.fill(q, t, d)
+                    case = "fill %s %s %d %dx%d" % (gi, ge, at, Lq, Lt)
                     for fast in (False, True):
                         s, pq, pt = O.fill(q, t, d, True, fast)
-                        assert_matrix_equal("score", s, rs)
-                        assert_matrix_equal("pq", pq, rq)
-                        assert_matrix_equal("pt", pt, rt)
+                        ref.check(case, s, pq, pt)
                         cells += s.size
                     if at == po.LOCAL and (Lq == 0 or Lt == 0):
                         continue  # optimal.h:100 reads getCell(-1,-1) here: undefined behaviour in the reference
                     rc, pairs, sc = O.optimal(s, pq, pt, d)
-                    rrc, rpairs, rsc = R.optimal(q, t, d)
-                    assert (rc != 0) == (rrc != 0)
-                    if rc == 0:
-                        assert_matrix_equal("optimal", pairs, rpairs)
-                        assert sc == rsc
+                    ref.check("optimal of " + case, rc != 0, *((pairs, sc) if rc == 0 else ()))
+    ref.close()
     assert cells > 100000
 
 
@@ -205,25 +198,22 @@ def test_oracle_sub_rectangle_fill_matches_golden(golden_sub):
             assert_matrix_equal(name + tag + ".pt", pt, g[name + "." + tag + ".pt"].astype(np.int32))
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference library not built")
 def test_oracle_sub_rectangle_fill_matches_reference_random(blosum):
-    alpha, M = blosum
+    _, M = blosum
+    ref = ReferenceResults("test_oracle.py::test_oracle_sub_rectangle_fill_matches_reference_random")
     rng = np.random.default_rng(17)
     for gi, ge in [(12, 1), (4.73, 0.34)]:
         for at in MODES:
             O = po.Oracle(M, gi, ge, at)
-            R = po.Reference(alpha, M, gi, ge, at)
             for trial in range(12):
                 Lq, Lt = int(rng.integers(1, 30)), int(rng.integers(1, 30))
                 q, t = rand_pair(rng, Lq, Lt)
                 q0 = int(rng.integers(0, Lq + 1)); q1 = int(rng.integers(q0 + 1, Lq + 2))
                 t0 = int(rng.integers(0, Lt + 1)); t1 = int(rng.integers(t0 + 1, Lt + 2))
                 for d in (po.FWD, po.REV):
-                    rs, rq, rt = R.fill_sub(q, t, (q0, t0, q1, t1), d)
                     s, pq, pt = O.fill_sub(q, t, (q0, t0, q1, t1), d)
-                    assert_matrix_equal("score", s, rs)
-                    assert_matrix_equal("pq", pq, rq)
-                    assert_matrix_equal("pt", pt, rt)
+                    ref.check("fill_sub %s %d %dx%d" % (gi, at, Lq, Lt), s, pq, pt)
+    ref.close()
 
 
 def test_oracle_tabulated_gap_fill_matches_golden(golden_tab):
@@ -237,8 +227,8 @@ def test_oracle_tabulated_gap_fill_matches_golden(golden_tab):
             assert_matrix_equal(name + tag + ".pt", pt, g[name + "." + tag + ".pt"].astype(np.int32))
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference library not built")
 def test_oracle_tabulated_gap_fill_matches_reference_random(blosum):
+    ref = ReferenceResults("test_oracle.py::test_oracle_tabulated_gap_fill_matches_reference_random")
     rng = np.random.default_rng(29)
     for at in MODES:
         for gen in (po.hmap_like_tables, po.gn2_like_tables):
@@ -246,16 +236,13 @@ def test_oracle_tabulated_gap_fill_matches_reference_random(blosum):
                 Lq, Lt = int(rng.integers(0, 45)), int(rng.integers(0, 45))
                 sim, dt, it = gen(rng, Lq, Lt, at)
                 for d in (po.FWD, po.REV):
-                    want = po.reference_fill_tab(sim, dt, it, at == po.LOCAL, d)
                     got = po.Oracle.fill_tab(sim, dt, it, at == po.LOCAL, d)
-                    for a, b, nm in zip(got, want, ("score", "pq", "pt")):
-                        assert_matrix_equal(nm, a, b)
+                    ref.check("fill_tab %d %dx%d" % (at, Lq, Lt), *got)
     # tables tabulated from the affine AASubstitutionEval model reproduce the ordinary reference fill
-    alpha, M = blosum
+    _, M = blosum
     for at in MODES:
         gi, ge = 4.73, 0.34
         O = po.Oracle(M, gi, ge, at)
-        R = po.Reference(alpha, M, gi, ge, at)
         q, t = rand_pair(rng, 27, 22)
         sz1, sz2 = len(q) + 2, len(t) + 2
         dt = np.zeros((sz2, sz2), np.float32)
@@ -271,27 +258,29 @@ def test_oracle_tabulated_gap_fill_matches_reference_random(blosum):
             for t2 in range(1, sz2):
                 it[ln, t2] = 0 if (ifree and (t2 == 1 or t2 == sz2 - 1)) else pen(ln)
         for d in (po.FWD, po.REV):
-            want = R.fill(q, t, d)
             got = po.Oracle.fill_tab(O.sim(q, t), dt, it, at == po.LOCAL, d)
-            for a, b, nm in zip(got, want[:3], ("score", "pq", "pt")):
-                assert_matrix_equal("affine-as-table " + nm, a, b)
+            ref.check("affine-as-table %d" % at, *got)
+    ref.close()
 
 
 def _canon(alis):
     return sorted((s, tuple(map(tuple, p))) for s, p in alis)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference library not built")
+def _canon_arrays(alis):
+    return [(s, np.array(p, np.int64).reshape(-1, 2)) for s, p in _canon(alis)]
+
+
 def test_oracle_ucw_enumeration_matches_reference(blosum):
     # orc_ucw_enumerate == UnconstrainedNearOptimal::enumerate (ucw.h:63-191): same alignments, same fp32 scores
     # (the reference sorts its set at the end, so the comparison is on canonically sorted lists)
-    alpha, M = blosum
+    _, M = blosum
+    ref = ReferenceResults("test_oracle.py::test_oracle_ucw_enumeration_matches_reference")
     rng = np.random.default_rng(4)
     total = 0
     for at in (po.GLOBAL_LOCAL, po.GLOBAL, po.LOCAL_GLOBAL, po.SEMI_LOCAL):
         for gi, ge in ((12, 1), (3, 1)):
             O = po.Oracle(M, gi, ge, at)
-            R = po.Reference(alpha, M, gi, ge, at)
             for Lq, Lt, delta in ((20, 25, 0.3), (30, 30, 0.2), (12, 40, 0.5), (0, 4, 0.1), (5, 1, 0.1)):
                 q = rng.integers(0, 20, Lq).astype(np.uint8)
                 t = q.copy() if Lq == Lt else rng.integers(0, 20, Lt).astype(np.uint8)
@@ -300,23 +289,22 @@ def test_oracle_ucw_enumeration_matches_reference(blosum):
                 thr = O.threshold(float(F[-1, -1]), delta)
                 st, alis = O.ucw_enumerate(q, t, F, O.sim(q, t), thr, 100000)
                 assert st == 0
-                ref = R.ucw_alignments(q, t, delta, 100000)
-                assert _canon(alis) == _canon(ref), (at, gi, Lq, Lt)
+                ref.check("ucw %d %s %dx%d" % (at, gi, Lq, Lt), _canon_arrays(alis))
                 total += len(alis)
+    ref.close()
     assert total > 2000
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference library not built")
 def test_oracle_constrained_enumeration_matches_reference(blosum):
     # orc_cno_enumerate == ConstrainedNearOptimal::enumerate (cw.h:60-284) for all-true, striped, random and all-false
     # SuboptFlags; integer and default float scoring
-    alpha, M = blosum
+    _, M = blosum
+    ref = ReferenceResults("test_oracle.py::test_oracle_constrained_enumeration_matches_reference")
     rng = np.random.default_rng(12)
     total = 0
     for at in (po.GLOBAL, po.SEMI_LOCAL, po.GLOBAL_LOCAL):
         for gi, ge in ((3, 1), (4.73, 0.34)):
             O = po.Oracle(M, gi, ge, at)
-            R = po.Reference(alpha, M, gi, ge, at)
             for Lq, Lt, delta in ((30, 30, 0.25), (12, 40, 0.5), (33, 33, 0.2), (1, 4, 0.2), (0, 3, 0.2)):
                 q = rng.integers(0, 20, Lq).astype(np.uint8)
                 t = q.copy() if Lq == Lt else rng.integers(0, 20, Lt).astype(np.uint8)
@@ -326,29 +314,28 @@ def test_oracle_constrained_enumeration_matches_reference(blosum):
                 for flags in (None, (np.arange(Lt + 2) // 5) % 2, rng.integers(0, 2, Lt + 2), np.zeros(Lt + 2, int)):
                     st, alis = O.cno_enumerate(q, t, F, O.sim(q, t), thr, pq, pt, flags, 100000)
                     assert st == 0
-                    ref = R.ucw_alignments(q, t, delta, 100000, 1, flags)
-                    assert _canon(alis) == _canon(ref), (at, gi, Lq, Lt)
+                    ref.check("cno %d %s %dx%d" % (at, gi, Lq, Lt), _canon_arrays(alis))
                     total += len(alis)
+    ref.close()
     assert total > 1000
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference library not built")
 def test_oracle_user_limit_truncation_matches_reference(blosum):
     # ucw.h:72 hard-codes user_limit = 100000; beyond it every further branch() forces the optimal path (ucw.h:115-126).
     # A 26 x 26 related pair at delta 0.5 has 251972 near-optimal alignments; the reference returns 100075.
-    alpha, M = blosum
+    _, M = blosum
+    ref = ReferenceResults("test_oracle.py::test_oracle_user_limit_truncation_matches_reference")
     rng = np.random.default_rng(21)
     L = 26
     q = rng.integers(0, 20, L).astype(np.uint8)
     t = q.copy()
     t[::3] = rng.integers(0, 20, len(t[::3]))
     O = po.Oracle(M, 3, 1, po.SEMI_LOCAL)
-    R = po.Reference(alpha, M, 3, 1, po.SEMI_LOCAL)
     F, pq, pt = O.fill(q, t, po.FWD, True, fast=False)
     thr = O.threshold(float(F[-1, -1]), 0.5)
     st, alis = O.ucw_enumerate(q, t, F, O.sim(q, t), thr, 300000, pq, pt)
-    ref = R.ucw_alignments(q, t, 0.5, 300000)
-    assert st == 0 and len(alis) == len(ref) > 100000
-    assert _canon(alis) == _canon(ref)
+    assert st == 0 and len(alis) > 100000
+    ref.check("truncated ucw", len(alis), _canon_arrays(alis))
+    ref.close()
     st, full = O.ucw_enumerate(q, t, F, O.sim(q, t), thr, 300000, pq, pt, user_limit=10 ** 9)
     assert len(full) > 2 * len(alis)

@@ -2,8 +2,9 @@
 
 CPU part (no GPU): the host walk that aadp_batch_near_optimal_pruned runs over a GPU-filled pair
 (alignment_algos_b200/csrc/aadp_pruned.h, built into tests/cxx/libpruned_host.so) is driven with the oracle's forward
-matrix and compared with the REFERENCE's own KSConstrainedNearOptimal / CRConstrainedNearOptimal, compiled from the
-unmodified headers by oracle/ref_harness.cpp.  GPU part (-m gpu): the same comparison through the C ABI over a resident batch.
+matrix and compared with the results of the REFERENCE's own KSConstrainedNearOptimal / CRConstrainedNearOptimal (compiled
+from the unmodified headers by oracle/ref_harness.cpp), stored in tests/golden/reference_digests.json.  GPU part (-m gpu):
+the same comparison through the C ABI over a resident batch.
 
 Bar: identical alignment sets (pairs and fp32 scores).  The reference ranks branch candidates with std::sort /
 std::partial_sort on the score alone, so which of several equal-score candidates survive a cut is a property of the
@@ -16,7 +17,7 @@ import subprocess
 import numpy as np
 import pytest
 
-from util import po, HAVE_REF, ROOT
+from util import po, ROOT, ReferenceResults
 
 LIB = os.path.join(ROOT, "tests", "cxx", "libpruned_host.so")
 
@@ -74,43 +75,42 @@ def cases(rng):
             yield q, t, delta, flags
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference library not built")
+VARIANTS = {2: "kscw", 3: "crcw"}
+
+
 @pytest.mark.parametrize("variant", [2, 3], ids=["kscw", "crcw"])
 def test_host_walk_equals_reference(blosum, variant):
-    alpha, M = blosum
+    _, M = blosum
+    ref = ReferenceResults("test_pruned.py::test_host_walk_equals_reference[%s]" % VARIANTS[variant])
     L = _host_lib()
     rng = np.random.default_rng(31 + variant)
     total = multi = 0
     for at in (po.SEMI_LOCAL, po.GLOBAL, po.GLOBAL_LOCAL):
         for gi, ge in ((3, 1), (12, 1), (4.73, 0.34)):
             O = po.Oracle(M, gi, ge, at)
-            R = po.Reference(alpha, M, gi, ge, at)
             for q, t, delta, flags in cases(rng):
                 F, pq, pt = O.fill(q, t, po.FWD, True, fast=False)
                 for kl, sl, mo in ((16, 100, 0.30), (4, 100, 0.30), (16, 8, 0.5), (2, 100, 0.1)):
-                    ref = R.pruned_alignments(q, t, delta, variant, flags, kl, sl, mo)
                     got = host_walk(L, variant, q, t, F, pq, pt, O.sim(q, t), flags, gi, ge, at, delta, kl, sl, mo)
-                    assert len(got) == len(ref), (at, gi, len(q), len(t), kl, sl, mo, len(got), len(ref))
-                    assert sorted(s for s, _ in got) == sorted(s for s, _ in ref)  # score multiset: independent of tie order
-                    assert canon(got) == canon(ref), (at, gi, len(q), len(t), kl, sl, mo)
+                    ref.check("%d %s %dx%d %d %d %s" % (at, gi, len(q), len(t), kl, sl, mo), canon(got))
                     total += len(got)
                     multi += len(got) > 1
+    ref.close()
     assert total > 3000 and multi > 100
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not HAVE_REF, reason="reference library not built")
 @pytest.mark.parametrize("variant", [2, 3], ids=["kscw", "crcw"])
 def test_gpu_pruned_enumerators_equal_reference(blosum, variant):
     # aadp_batch_near_optimal_pruned over a resident batch (forward fill, traceback and scores produced by the CUDA
     # kernels; integer grid -> packed kernels, 4.73/0.34 -> exact general-gap kernel) against the reference's own
     # KSConstrainedNearOptimal / CRConstrainedNearOptimal
     import alignment_algos_b200 as a
-    alpha, M = blosum
+    _, M = blosum
+    ref = ReferenceResults("test_pruned.py::test_gpu_pruned_enumerators_equal_reference[%s]" % VARIANTS[variant])
     rng = np.random.default_rng(41 + variant)
     total = 0
     for at, gi, ge in ((po.SEMI_LOCAL, 3, 1), (po.GLOBAL, 12, 1), (po.GLOBAL_LOCAL, 4.73, 0.34)):
-        R = po.Reference(alpha, M, gi, ge, at)
         cs = list(cases(rng))
         seqs, pq, pt = [], [], []
         for q, t, delta, flags in cs:
@@ -122,14 +122,13 @@ def test_gpu_pruned_enumerators_equal_reference(blosum, variant):
         c.fill_batch(res, off, np.array(pq, np.int32), np.array(pt, np.int32), a.W_FWD | a.W_TB | a.W_SCORES, 0.1)
         for p, (q, t, delta, flags) in enumerate(cs):
             for kl, sl, mo in ((16, 100, 0.30), (4, 8, 0.5)):
-                ref = R.pruned_alignments(q, t, delta, variant, flags, kl, sl, mo)
                 st, thr, got = c.near_optimal_pruned(p, variant, delta, len(q), len(t), flags, kl, sl, mo)
                 assert st == 0
-                assert sorted(s for s, _ in got) == sorted(s for s, _ in ref), (at, gi, p, kl)
-                assert canon(got) == canon(ref), (at, gi, p, kl)
+                ref.check("%d %s pair %d %d" % (at, gi, p, kl), canon(got))
                 total += len(got)
         # a budget smaller than the set: status 1
         st, _, got = c.near_optimal_pruned(1, 2, cs[1][2], len(cs[1][0]), len(cs[1][1]), cs[1][3], max_alignments=1)
         assert st in (0, 1) and len(got) <= 1
         c.close()
+    ref.close()
     assert total > 500
