@@ -1620,18 +1620,28 @@ static int gg_fill(aadp_ctx* c, int64_t p0, int64_t n, int dirmask, bool tb, con
   // ids != nullptr: the n items are the listed pairs ids[0..n) instead of the consecutive pairs p0..p0+n
   Batch& b = c->b;
   const int64_t cells = off[(size_t)n];
-  int maxLt = 0, maxL = 0;
+  // What the kernels keep per item in shared memory is indexed by flow column (at most nt, the interior columns) and by
+  // gap length (at most max(nq, nt)): for a whole matrix nt = Lt and nq = Lq, for a sub-rectangle only the rectangle
+  // counts, however long its sequences are.  The widest item picks the kernel, its variant and the shared memory.
+  int maxNt = 0, maxLen = 0;
   for (int64_t k = 0; k < n; ++k) {
-    const int64_t p = ids ? ids[k] : p0 + k;
-    const int qs = b.pair_q[p], ts = b.pair_t[p];
-    const int Lq = (int)(b.seq_off[qs + 1] - b.seq_off[qs]), Lt = (int)(b.seq_off[ts + 1] - b.seq_off[ts]);
-    maxLt = std::max(maxLt, Lt);
-    maxL = std::max(maxL, std::max(Lq, Lt));
+    int nq, nt;
+    if (rect) {
+      nq = rect[4 * k + 2] - rect[4 * k] - 1;
+      nt = rect[4 * k + 3] - rect[4 * k + 1] - 1;
+    } else {
+      const int64_t p = ids ? ids[k] : p0 + k;
+      const int qs = b.pair_q[p], ts = b.pair_t[p];
+      nq = (int)(b.seq_off[qs + 1] - b.seq_off[qs]);
+      nt = (int)(b.seq_off[ts + 1] - b.seq_off[ts]);
+    }
+    maxNt = std::max(maxNt, nt);
+    maxLen = std::max(maxLen, std::max(nq, nt));
   }
-  const size_t smem = (size_t)(2 * (maxLt + 2) + maxL + 2 + 32) * sizeof(float);
+  const size_t smem = (size_t)(2 * (maxNt + 2) + maxLen + 2 + 32) * sizeof(float);
   if (smem > 220 * 1024) return fail("exact general-gap path: sequences too long for the shared-memory row and penalty tables");
   // the pruned scans (prefix maxima + binary searches) only pay off when the scans are long
-  int longest = maxL;
+  int longest = maxLen;
   if (rect) {
     longest = 1;
     for (int64_t k = 0; k < n; ++k)
@@ -1639,10 +1649,12 @@ static int gg_fill(aadp_ctx* c, int64_t p0, int64_t n, int dirmask, bool tb, con
   }
   const bool prune_pays = longest >= 96;
   // record-list kernel (aadp_frec.cuh): affine gaps only; one warp per (pair, direction), rows and column leaders in
-  // shared memory, 16-bit row/column indices
-  const int rec_cap = frec_cap(maxLt);
-  const bool use_rec = c->gg_records && !(ov && ov->d_del) && maxL < 32000 && maxLt <= 2048 && frec_smem_bytes(rec_cap) <= 200 * 1024;
+  // shared memory, 16-bit flow row/column indices, at most 64 key columns per lane
+  const int rec_cap = frec_cap(maxNt);
+  const bool use_rec = c->gg_records && !(ov && ov->d_del) && maxLen < 32000 && maxNt <= 2048 && frec_smem_bytes(rec_cap) <= 200 * 1024;
   GeneralParams G{};
+  G.max_nt = maxNt;
+  G.max_len = maxLen;
   G.A = c->sc.A;
   G.subf = c->subf.as<float>();
   G.gi = c->gi_f;
@@ -1714,14 +1726,11 @@ static int gg_fill(aadp_ctx* c, int64_t p0, int64_t n, int dirmask, bool tb, con
   }
   G.compact = compact ? 1 : 0;      // compact batches (aadp_fill_subpair_batch) keep only the rectangles and
   G.fin_by_item = compact ? 1 : 0;  // index the final scores by item: several items may share one pair
-  int width = maxLt;  // threads own columns: of the matrix, or of the widest rectangle
+  const int width = rect ? std::max(1, maxNt) : maxNt;  // threads own columns: of the matrix, or of the widest rectangle
   double cu = 0;
   if (rect) {
-    width = 1;
-    for (int64_t k = 0; k < n; ++k) {
-      width = std::max(width, rect[4 * k + 3] - rect[4 * k + 1] - 1);
+    for (int64_t k = 0; k < n; ++k)
       cu += (double)(rect[4 * k + 2] - rect[4 * k] - 1) * (double)(rect[4 * k + 3] - rect[4 * k + 1] - 1);
-    }
   } else {
     for (int64_t k = 0; k < n; ++k) {
       const int64_t p = ids ? ids[k] : p0 + k;
@@ -1732,13 +1741,15 @@ static int gg_fill(aadp_ctx* c, int64_t p0, int64_t n, int dirmask, bool tb, con
   // few CTAs (single pairs): latency counts, one column per thread; many CTAs: smaller CTAs hide each other's barriers
   const int tcap = n * nd < 296 ? 512 : c->gg_threads_cap;
   const int threads = std::max(compact ? 32 : 64, std::min(tcap, (width + 31) / 32 * 32));
-  c->prof_begin(use_rec ? (tb ? "frec_fill_kernel<TB=1>" : "frec_fill_kernel<TB=0>")
+  const bool wide = maxNt > 1024;  // record-list kernel: more than 32 key columns per lane
+  static const char* const kFrecNames[2][2] = {{"frec_fill_kernel<TB=0>", "frec_fill_kernel<TB=0,WIDE=1>"},
+                                               {"frec_fill_kernel<TB=1>", "frec_fill_kernel<TB=1,WIDE=1>"}};
+  c->prof_begin(use_rec ? kFrecNames[tb][wide]
                         : tab ? "general_fill_kernel<TB=1,TAB=1>" : tb ? "general_fill_kernel<TB=1>" : "general_fill_kernel<TB=0>", cu * nd);
   if (use_rec) {
     // (measurement aid: AADP_FREC_SMEM_PAD extra bytes per warp lower the resident warps per SM)
     const size_t rsm = frec_smem_bytes(rec_cap) + (getenv("AADP_FREC_SMEM_PAD") ? (size_t)atoi(getenv("AADP_FREC_SMEM_PAD")) : 0);
     const dim3 grid((unsigned)n, (unsigned)nd);
-    const bool wide = maxLt > 1024;  // more than 32 key columns per lane
 #define AADP_FREC_LAUNCH(TB_, WIDE_)                                                      \
     do {                                                                                  \
       CK(cached_max_smem((const void*)frec_fill_kernel<TB_, WIDE_>, rsm));               \

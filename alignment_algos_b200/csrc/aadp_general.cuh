@@ -54,7 +54,10 @@ struct GeneralParams {
                              // first anchor at offset 0 (batched loop-closure fills: many small rectangles of large
                              // matrices); predecessors stay matrix indices
   int fin_by_item;           // 1: fin[] is indexed by item0 + item instead of by pair
-  float* score[2];           // per direction: dense score matrices (always)
+  int max_nt;                // launch-wide shared-memory layout (general_fill_kernel): the most interior columns of an
+  int max_len;               // item and the longest gap an item can take, max(nq, nt) -- for sub-rectangles those of the
+                             // rectangles, not of the sequences (a loop in a 30 000-residue pair needs a few hundred floats)
+  float* score[2];          // per direction: dense score matrices (always)
   int32_t* prevq[2];         // per direction: dense predecessor rows/cols, or null
   int32_t* prevt[2];
   float* fin[2];             // per direction, per PAIR: score of the final cell, or null
@@ -110,10 +113,11 @@ __global__ void __launch_bounds__(512) general_fill_kernel(const GeneralParams P
   const float gi = P.gi, ge = P.ge;
   const bool local = P.local != 0;
 
-  float* prow = gg_smem;              // D[a-1][0..nt]
-  float* pen = gg_smem + (Lt + 2);    // pen[len], len >= 1
-  float* pm = pen + (max(Lq, Lt) + 2);  // pm[k] = max(prow[1..k])  (pruned scans)
-  float* wmax = pm + (Lt + 2);          // 32 warp maxima of the block-wide prefix scan
+  // indexed by flow column (prow, pm) and by gap length (pen): sized by the launch (nt <= max_nt, max(nq, nt) <= max_len)
+  float* prow = gg_smem;                // D[a-1][0..nt]
+  float* pen = gg_smem + (P.max_nt + 2);  // pen[len], len >= 1
+  float* pm = pen + (P.max_len + 2);    // pm[k] = max(prow[1..k])  (pruned scans)
+  float* wmax = pm + (P.max_nt + 2);    // 32 warp maxima of the block-wide prefix scan
   const bool PRUNE = !TAB && P.pmcol[dsel] != nullptr;
   float* PMC = PRUNE ? P.pmcol[dsel] + base : nullptr;
   const float* del_tab = TAB ? P.del_tab + (P.del_off ? P.del_off[item] : 0) : nullptr;

@@ -113,8 +113,11 @@ int aadp_fill_pair(aadp_ctx* ctx, const uint8_t* q, int Lq, const uint8_t* t, in
  * (q1_end, t1_end) and (q2_beg, t2_beg) (matrix indices, 0 = Head, L+1 = Tail); both anchor scores are 0,
  * cells outside the rectangle keep the DPCell defaults (score 0, predecessors -1).  Anchors that are ordinary
  * residues pay gap penalties and the final cell adds its real similarity, exactly as the reference does.
- * Always computed by the exact general-gap fp32 kernel (any scoring).  direction: AADP_FWD or AADP_REV.
- * Outputs are (Lq+2)*(Lt+2) host arrays, any may be NULL.                                                 */
+ * Always computed by an exact fp32 kernel (any scoring): the record-list kernel (frec_fill_kernel) by default, the
+ * general-gap kernel (general_fill_kernel) with option general_records 0 or beyond the record-list kernel's limits (more
+ * than 2048 interior columns, or 32 000 interior rows).  The rectangle alone picks the kernel and sizes its shared
+ * memory, not the sequence lengths.
+ * direction: AADP_FWD or AADP_REV.  Outputs are (Lq+2)*(Lt+2) host arrays, any may be NULL.               */
 int aadp_fill_subpair(aadp_ctx* ctx, const uint8_t* q, int Lq, const uint8_t* t, int Lt, int q1_end,
                       int t1_end, int q2_beg, int t2_beg, int direction, float* score,
                       int32_t* prev_q, int32_t* prev_t);
@@ -124,8 +127,10 @@ int aadp_fill_subpair(aadp_ctx* ctx, const uint8_t* q, int Lq, const uint8_t* t,
  * followed by Optimal_Subali::enumerate (optimal_subali.h:59-83) -- for a whole list of loops.
  * Item k fills the rectangle rects[4k..4k+3] = (q1_end, t1_end, q2_beg, t2_beg) of query sequence item_q[k] against
  * template sequence item_t[k] (ids into residues/seq_off as in aadp_fill_batch; items may share sequences).  Each
- * item runs on the exact general-gap fp32 kernel in COMPACT storage: only its rectangle lives in HBM, not the
- * (Lq+2)*(Lt+2) matrix around it.  direction: AADP_FWD or AADP_REV (REV: scores only).  Host outputs (any may be NULL):
+ * item runs on an exact fp32 kernel as in aadp_fill_subpair, in COMPACT storage: only its rectangle lives on the
+ * device, in HBM and in shared memory, not the (Lq+2)*(Lt+2) matrix around it, so loops of very long pairs fill too.
+ * Items are launched in chunks (option general_budget_mcells); the widest rectangle of a chunk picks its kernel, and
+ * every result is the same whatever chunk an item lands in.  direction: AADP_FWD or AADP_REV (REV: scores only).  Host outputs (any may be NULL):
  *   score    nitems: score of the final cell, D[q2_beg][t2_beg] (FWD, = AlignedPairList::score of
  *            optimal_subali.h:68) or D[q1_end][t1_end] (REV)
  *   ali_off  nitems+1: slot k is ali_off[k]..ali_off[k+1] = q2_beg-q1_end+1 aligned pairs (every traceback step lowers

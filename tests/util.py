@@ -113,3 +113,15 @@ def assert_matrix_equal(name, got, want):
     bad = np.argwhere(got != want)
     assert len(bad) == 0, "%s: %d mismatching cells, first at %s: got %s want %s" % (
         name, len(bad), tuple(bad[0]), got[tuple(bad[0])], want[tuple(bad[0])])
+
+
+def subali_walk(S, PQ, PT, rect):
+    """Optimal_Subali::enumerate (optimal_subali.h:59-83) over reference-shaped dense matrices: (status, aligned pairs
+    from (q1_end, t1_end) to (q2_beg, t2_beg), score of the final cell)."""
+    q1, t1, q2, t2 = [int(x) for x in rect]
+    i, j = q2, t2
+    path = [(i, j)]
+    while i > q1:
+        i, j = int(PQ[i, j]), int(PT[i, j])
+        path.insert(0, (i, j))
+    return (0 if (i, j) == (q1, t1) else 3), np.array(path, np.int32).reshape(-1, 2), S[q2, t2]
