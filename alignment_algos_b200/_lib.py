@@ -36,6 +36,7 @@ def lib():
     L.aadp_synchronize.argtypes = [vp]
     L.aadp_set_option.argtypes = [vp, cp, C.c_int]
     L.aadp_set_scoring.argtypes = [vp, vp, C.c_int, f32, f32, C.c_int, u32]
+    L.aadp_set_profile_scoring.argtypes = [vp, vp, vp, i64, C.c_int, f32, f32, C.c_int, u32]
     L.aadp_fill_pair.argtypes = [vp, vp, C.c_int, vp, C.c_int, C.c_int, f32] + [vp] * 8
     L.aadp_fill_batch.argtypes = [vp, vp, vp, i64, vp, vp, i64, u32, f32, vp, vp, vp, vp]
     L.aadp_fill_batch_submit.argtypes = [vp, vp, vp, i64, vp, vp, i64, u32, f32, vp, vp, vp, vp]
@@ -84,7 +85,7 @@ def lib():
 
 EXPORTS = [
     "aadp_create", "aadp_destroy", "aadp_last_error", "aadp_version", "aadp_set_stream",
-    "aadp_synchronize", "aadp_set_option", "aadp_set_scoring", "aadp_fill_pair", "aadp_fill_batch",
+    "aadp_synchronize", "aadp_set_option", "aadp_set_scoring", "aadp_set_profile_scoring", "aadp_fill_pair", "aadp_fill_batch",
     "aadp_upload_batch", "aadp_run_batch", "aadp_batch_resident_bytes", "aadp_last_launch_count",
     "aadp_last_h2d_bytes", "aadp_last_d2h_bytes", "aadp_last_cell_updates", "aadp_set_profiling", "aadp_profile_count", "aadp_profile_get",
     "aadp_batch_fetch_pair", "aadp_batch_optimal", "aadp_tb_row_bytes", "aadp_batch_tb_bytes",

@@ -66,6 +66,28 @@ class Context:
         self._ck(self.L.aadp_set_scoring(self.h, _ptr(sub), sub.shape[0], gi, ge, align_type, flags))
         self.align_type, self.flags = align_type, flags
 
+    @staticmethod
+    def pack_profiles(profiles):
+        """Position-specific template profiles, indexed by sequence id: an (L, A) array per sequence (row j-1 = the scores
+        of query codes 0..A-1 against template position j) or None for a sequence that is only ever a query.
+        Returns (prof float32[total], prof_off int64[n+1], A) as aadp_set_profile_scoring takes them."""
+        arrs = [None if p is None else np.asarray(p, np.float32) for p in profiles]
+        widths = {a.shape[1] for a in arrs if a is not None and a.ndim == 2}
+        if any(a is not None and a.ndim != 2 for a in arrs) or len(widths) != 1:
+            raise ValueError("profiles: (L, A) arrays with one A for every sequence (None for query-only sequences)")
+        A = widths.pop()
+        off = np.zeros(len(arrs) + 1, np.int64)
+        off[1:] = np.cumsum([0 if a is None else a.size for a in arrs])
+        data = [a.ravel() for a in arrs if a is not None and a.size]
+        prof = np.ascontiguousarray(np.concatenate(data) if data else np.zeros(0, np.float32), np.float32)
+        return prof, off, A
+
+    def set_profile_scoring(self, profiles, gi, ge, align_type, flags=REPRO_REV_BUG):
+        """aadp_set_profile_scoring: a pair with template sequence t scores sim(i, j) = profiles[t][j-1, q_i]."""
+        prof, off, A = self.pack_profiles(profiles)
+        self._ck(self.L.aadp_set_profile_scoring(self.h, _ptr(prof), _ptr(off), len(off) - 1, A, gi, ge, align_type, flags))
+        self.align_type, self.flags = align_type, flags
+
     # ---- single pair (DPMatrix constructor replacement) ----
     def fill_pair(self, q, t, direction=FWD, delta_ratio=-1.0, want_tb=True, want_scores=True):
         q = np.ascontiguousarray(q, dtype=np.uint8)

@@ -145,6 +145,15 @@ struct aadp_ctx {
   std::vector<float> subf_h;  // the substitution table as given (host copy: similarity matrix of the pruned enumerators)
   int max_abs_sub = 0;
   DevBuf sub8p;
+  // position-specific template profiles (aadp_set_profile_scoring): replace sub8 / sub8p / subf while prof_mode is set
+  bool prof_mode = false;
+  int64_t prof_nseq = 0;              // profiles given (one per sequence id)
+  std::vector<int64_t> prof_len;      // per sequence: entries (L*A), 0 = no profile
+  std::vector<int> prof_max;          // per sequence: max |entry| in grid units (the per-template score bound)
+  std::vector<float> proff_h;         // the profiles as given (host copy: similarity matrix of the pruned enumerators)
+  std::vector<int64_t> proff_off_h;
+  DevBuf prof8, prof8_off, proff, proff_off;
+  ProfDev prof_dev() const { return ProfDev{prof8.as<int8_t>(), prof8_off.as<int64_t>(), proff.as<float>(), proff_off.as<int64_t>()}; }
   DevBuf sub8, residues, seq_off, pair_q, pair_t, order[2], tb_off, sc_off, mask_off;
   DevBuf tb[2], scb[2], mask, fin_score[2], fin_kind[2], fin_k[2], counter, bbuf, thr, count, fscore[2];
   DevBuf scratch_a, scratch_b, scratch_c, scratch_d;
@@ -257,9 +266,9 @@ struct TimeMarks {
 };
 thread_local TimeMarks g_marks;
 
-template <int K, int TBM, int STM>
+template <int K, int TBM, int STM, int PRO>
 int launch_fill_t(aadp_ctx* c, FillParams& P) {
-  auto kern = fill_kernel<K, TBM, STM>;
+  auto kern = fill_kernel<K, TBM, STM, PRO>;
   const int A = P.sc.A;
   const size_t smem = (size_t)((A * A + 15) / 16 * 16) + (size_t)kWarpsPerCta * (kQRing + A * 32 * K);
   CK(cached_max_smem((const void*)kern, (size_t)(smem)));
@@ -278,25 +287,29 @@ int launch_fill_t(aadp_ctx* c, FillParams& P) {
     P.bb_rows = c->bb_rows;
   }
   char nm[64];
-  snprintf(nm, sizeof nm, "fill_kernel<K=%d,TB=%d,ST=%d>%s", K, TBM, STM, P.rev ? "rev" : "fwd");
+  snprintf(nm, sizeof nm, "fill_kernel<K=%d,TB=%d,ST=%d%s>%s", K, TBM, STM, PRO ? ",PRO=1" : "", P.rev ? "rev" : "fwd");
   c->prof_begin(nm, P.cells_hint);
-  kern<<<grid, kWarpsPerCta * 32, smem, c->stream>>>(P);
+  kern<<<grid, kWarpsPerCta * 32, smem, c->stream>>>(P, c->prof_dev());
   c->prof_end();
   CK(cudaGetLastError());
   c->launches++;
   return 0;
 }
 
+template <int K, int PRO>
+int launch_fill_kp(aadp_ctx* c, FillParams& P, int tbm, int stm) {
+  if (tbm == 0) {
+    if (stm == 0) return launch_fill_t<K, 0, 0, PRO>(c, P);
+    if (stm == 1) return launch_fill_t<K, 0, 1, PRO>(c, P);
+    return launch_fill_t<K, 0, 2, PRO>(c, P);
+  }
+  if (stm == 0) return launch_fill_t<K, 1, 0, PRO>(c, P);
+  if (stm == 1) return launch_fill_t<K, 1, 1, PRO>(c, P);
+  return launch_fill_t<K, 1, 2, PRO>(c, P);
+}
 template <int K>
 int launch_fill_k(aadp_ctx* c, FillParams& P, int tbm, int stm) {
-  if (tbm == 0) {
-    if (stm == 0) return launch_fill_t<K, 0, 0>(c, P);
-    if (stm == 1) return launch_fill_t<K, 0, 1>(c, P);
-    return launch_fill_t<K, 0, 2>(c, P);
-  }
-  if (stm == 0) return launch_fill_t<K, 1, 0>(c, P);
-  if (stm == 1) return launch_fill_t<K, 1, 1>(c, P);
-  return launch_fill_t<K, 1, 2>(c, P);
+  return c->prof_mode ? launch_fill_kp<K, 1>(c, P, tbm, stm) : launch_fill_kp<K, 0>(c, P, tbm, stm);
 }
 
 // Builds the 16-byte aligned forward and reversed sequence arenas on the device and validates the
@@ -317,9 +330,9 @@ __global__ void arena_kernel(const uint8_t* __restrict__ res, const int64_t* __r
   }
 }
 
-template <int TBM, int FST, int MSK, int LOC = 0>
+template <int TBM, int FST, int MSK, int LOC = 0, int PRO = 0>
 int launch_packed_t(aadp_ctx* c, PackedParams& P) {
-  auto kern = packed_kernel<TBM, FST, MSK, 0, LOC>;
+  auto kern = packed_kernel<TBM, FST, MSK, 0, LOC, PRO>;
   const int A = P.sc.A;
   size_t smem = packed_smem_bytes(A, MSK);
   // measurement aid: AADP_PACKED_SMEM_PAD="fwd,rev" extra bytes per CTA lower the resident warps per SM
@@ -336,8 +349,10 @@ int launch_packed_t(aadp_ctx* c, PackedParams& P) {
   if (grid > need) grid = need;
   if (grid < 1) grid = 1;
   char nm[64];
-  snprintf(nm, sizeof nm, "packed_kernel<TB=%d,FST=%d,MSK=%d%s>%s", TBM, FST, MSK, LOC ? ",LOC=1" : "", P.rev ? "rev" : "fwd");
+  snprintf(nm, sizeof nm, "packed_kernel<TB=%d,FST=%d,MSK=%d%s%s>%s", TBM, FST, MSK, LOC ? ",LOC=1" : "", PRO ? ",PRO=1" : "",
+           P.rev ? "rev" : "fwd");
   c->prof_begin(nm, P.cells_hint);
+  P.prof = c->prof_dev();
   kern<<<grid, kPackedWarps * 32, smem, c->stream>>>(P);
   c->prof_end();
   CK(cudaGetLastError());
@@ -345,27 +360,31 @@ int launch_packed_t(aadp_ctx* c, PackedParams& P) {
   return 0;
 }
 
-int launch_packed(aadp_ctx* c, PackedParams& P, int tbm, int fst, int msk) {
+template <int PRO>
+int launch_packed_p(aadp_ctx* c, PackedParams& P, int tbm, int fst, int msk) {
   const int key = tbm * 4 + fst * 2 + msk;
   if (P.sc.local) {  // local alignments: the clamped variants (never with the fused near-optimal pass)
     if (msk) return fail("internal: local alignments have no fused near-optimal pass");
     switch (key) {
-      case 0: return launch_packed_t<0, 0, 0, 1>(c, P);
-      case 2: return launch_packed_t<0, 1, 0, 1>(c, P);
-      case 4: return launch_packed_t<1, 0, 0, 1>(c, P);
-      default: return launch_packed_t<1, 1, 0, 1>(c, P);
+      case 0: return launch_packed_t<0, 0, 0, 1, PRO>(c, P);
+      case 2: return launch_packed_t<0, 1, 0, 1, PRO>(c, P);
+      case 4: return launch_packed_t<1, 0, 0, 1, PRO>(c, P);
+      default: return launch_packed_t<1, 1, 0, 1, PRO>(c, P);
     }
   }
   switch (key) {
-    case 0: return launch_packed_t<0, 0, 0>(c, P);
-    case 1: return launch_packed_t<0, 0, 1>(c, P);
-    case 2: return launch_packed_t<0, 1, 0>(c, P);
-    case 3: return launch_packed_t<0, 1, 1>(c, P);
-    case 4: return launch_packed_t<1, 0, 0>(c, P);
-    case 5: return launch_packed_t<1, 0, 1>(c, P);
-    case 6: return launch_packed_t<1, 1, 0>(c, P);
-    default: return launch_packed_t<1, 1, 1>(c, P);
+    case 0: return launch_packed_t<0, 0, 0, 0, PRO>(c, P);
+    case 1: return launch_packed_t<0, 0, 1, 0, PRO>(c, P);
+    case 2: return launch_packed_t<0, 1, 0, 0, PRO>(c, P);
+    case 3: return launch_packed_t<0, 1, 1, 0, PRO>(c, P);
+    case 4: return launch_packed_t<1, 0, 0, 0, PRO>(c, P);
+    case 5: return launch_packed_t<1, 0, 1, 0, PRO>(c, P);
+    case 6: return launch_packed_t<1, 1, 0, 0, PRO>(c, P);
+    default: return launch_packed_t<1, 1, 1, 0, PRO>(c, P);
   }
+}
+int launch_packed(aadp_ctx* c, PackedParams& P, int tbm, int fst, int msk) {
+  return c->prof_mode ? launch_packed_p<1>(c, P, tbm, fst, msk) : launch_packed_p<0>(c, P, tbm, fst, msk);
 }
 
 // shared memory of a wavefront CTA (one warp = one stripe): substitution table, query ring + staging block, profile
@@ -374,7 +393,8 @@ static size_t wave_smem_bytes(int A) {
 }
 // CTAs of the wavefront kernel that can be resident at once (all stripes of a pair wait on each other)
 static int wave_resident_ctas(aadp_ctx* c, int A) {
-  auto kern = wave_kernel<kWaveK, 1, 2>;  // the largest variant
+  // the largest variant
+  const void* kern = c->prof_mode ? (const void*)wave_kernel<kWaveK, 1, 2, 1> : (const void*)wave_kernel<kWaveK, 1, 2, 0>;
   const size_t smem = wave_smem_bytes(A);
   if (cached_max_smem((const void*)kern, smem) != cudaSuccess) return 0;
   int occ = 0;
@@ -384,7 +404,8 @@ static int wave_resident_ctas(aadp_ctx* c, int A) {
 
 template <int TBM, int STM>
 int launch_wave_t(aadp_ctx* c, FillParams& Pf, FillParams& Pr, int ndirs, int nst) {
-  auto kern = wave_kernel<kWaveK, TBM, STM>;
+  const bool pro = c->prof_mode;
+  const void* kern = pro ? (const void*)wave_kernel<kWaveK, TBM, STM, 1> : (const void*)wave_kernel<kWaveK, TBM, STM, 0>;
   const int A = Pf.sc.A;
   const size_t smem = wave_smem_bytes(A);
   CK(cached_max_smem((const void*)kern, (size_t)(smem)));
@@ -393,10 +414,11 @@ int launch_wave_t(aadp_ctx* c, FillParams& Pf, FillParams& Pr, int ndirs, int ns
   const int grid = ndirs * nst;
   if (occ < 1 || grid > occ * c->num_sms) return fail("wavefront kernel: stripes of this pair cannot all be resident");
   char nm[64];
-  snprintf(nm, sizeof nm, "wave_kernel<K=%d,TB=%d,ST=%d>x%d", kWaveK, TBM, STM, ndirs);
+  snprintf(nm, sizeof nm, "wave_kernel<K=%d,TB=%d,ST=%d%s>x%d", kWaveK, TBM, STM, pro ? ",PRO=1" : "", ndirs);
   c->prof_begin(nm, Pf.cells_hint * ndirs);
   int nd = ndirs;
-  void* args[] = {(void*)&Pf, (void*)&Pr, (void*)&nd};
+  ProfDev pd = c->prof_dev();
+  void* args[] = {(void*)&Pf, (void*)&Pr, (void*)&nd, (void*)&pd};
   CK(cudaLaunchCooperativeKernel((void*)kern, dim3(grid), dim3(32), args, smem, c->stream));
   c->prof_end();
   c->launches++;
@@ -574,6 +596,22 @@ void build_tasks_range(const Batch& b, const int32_t* Lq32, const int32_t* Lt32,
   }
 }
 
+// Profile scoring: one profile per sequence id of the batch, and a template's profile must hold L_t*A entries.
+int profile_count_refusal(aadp_ctx* c, int64_t nseq) {
+  if (c->prof_nseq >= nseq) return 0;
+  return fail("profile scoring: " + std::to_string(c->prof_nseq) + " profiles for " + std::to_string(nseq) +
+              " sequences; aadp_set_profile_scoring needs one profile (possibly empty) per sequence id");
+}
+int profile_refusal(aadp_ctx* c, int64_t ts, int64_t Lt) {
+  const int64_t n = c->prof_len[(size_t)ts];
+  if (n == 0)
+    return fail("profile scoring: sequence " + std::to_string(ts) + " is used as a template (" + std::to_string(Lt) +
+                " residues) but its profile is empty");
+  return fail("profile scoring: the profile of sequence " + std::to_string(ts) + " has " + std::to_string(n) +
+              " entries, but the template has " + std::to_string(Lt) + " residues: L*A = " + std::to_string(Lt * c->sc.A) +
+              " entries are needed");
+}
+
 // Classifies every pair (packed / int32 / wavefront), sizes its resident products and builds the packed
 // task list.  All O(npairs) passes run on `host_threads` threads over disjoint pair ranges; the per-range
 // task lists (each longest first) are interleaved round-robin so the global order stays longest first.
@@ -606,8 +644,10 @@ int build_batch_meta(aadp_ctx* c, uint32_t what) {
   c->Lt32.resize((size_t)np);
   int32_t* const Lq32 = c->Lq32.data();
   int32_t* const Lt32 = c->Lt32.data();
+  if (c->prof_mode && profile_count_refusal(c, b.nseq)) return 1;
   struct Part {
     int err = 0, max_Lq = 0, max_Lt = 0;
+    int64_t bad_seq = 0;
     int64_t bound = 0, sum[3] = {0, 0, 0};
     double cells = 0, packed_cells = 0, bucket_cells[2] = {0, 0};
   };
@@ -634,8 +674,14 @@ int build_batch_meta(aadp_ctx* c, uint32_t what) {
       P.max_Lt = std::max<int>(P.max_Lt, (int)Lt);
       const int64_t cl = Lq * Lt;
       P.cells += (double)cl;
+      // |similarity| bound: the substitution table's, or (profile scoring) the template's own
+      int64_t mx = c->max_abs_sub;
+      if (c->prof_mode) {
+        if (c->prof_len[(size_t)ts] != Lt * c->sc.A) { P.err = 3; P.bad_seq = ts; break; }
+        mx = c->prof_max[(size_t)ts];
+      }
       // |score| bound in integer units: matches + one end gap on each side
-      const int64_t bd = std::min(Lq, Lt) * (int64_t)c->max_abs_sub + 2 * (int64_t)c->sc.gi + (int64_t)c->sc.ge * (Lq + Lt);
+      const int64_t bd = std::min(Lq, Lt) * mx + 2 * (int64_t)c->sc.gi + (int64_t)c->sc.ge * (Lq + Lt);
       // (local alignments: the packed kernel has no fused near-optimal pass for them -- F + R - sim needs both clamped
       // matrices -- so a local run that asks for the cell set keeps the int32 kernels + mask_kernel)
       const bool packed_ok = c->allow_packed && (!c->sc.local || !(what & AADP_W_MASK)) && Lq >= 1 && Lt >= 1 && Lt <= 512 && bd < kPackedBound &&
@@ -665,6 +711,7 @@ int build_batch_meta(aadp_ctx* c, uint32_t what) {
     const SchedScratch& S = c->sched[(size_t)t];
     if (P.err == 1) return fail("pair index out of range");
     if (P.err == 2) return fail("bad sequence length");
+    if (P.err == 3) return profile_refusal(c, P.bad_seq, b.seq_off[(size_t)P.bad_seq + 1] - b.seq_off[(size_t)P.bad_seq]);
     b.max_Lq = std::max(b.max_Lq, P.max_Lq);
     b.max_Lt = std::max(b.max_Lt, P.max_Lt);
     b.cells += P.cells;
@@ -1122,7 +1169,8 @@ void aadp_destroy(aadp_ctx* c) {
                    &c->x_layout, &c->x_qc, &c->x_qid, &c->x_tid, &c->x_scores,
                    &c->subf, &c->gg_score[0], &c->gg_score[1], &c->gg_pq[0], &c->gg_pq[1], &c->gg_pt[0], &c->gg_pt[1],
                    &c->gg_mask, &c->gg_off, &c->gg_fin[0], &c->gg_fin[1], &c->gg_pm[0], &c->gg_pm[1], &c->gg_items, &c->tb_del, &c->tb_ins, &c->tb_del_off, &c->tb_ins_off, &c->ali_cap, &c->ali_out, &c->ali_n, &c->ali_status, &c->gg_rect, &c->sub8p,
-                   &c->ucw_ids, &c->ucw_path_off, &c->ucw_stack_off, &c->ucw_stack, &c->ucw_paths, &c->ucw_len, &c->ucw_scores, &c->ucw_n, &c->ucw_status, &c->ucw_thr, &c->ucw_plen, &c->ucw_pathbuf, &c->ucw_flags, &c->ucw_flag_off};
+                   &c->ucw_ids, &c->ucw_path_off, &c->ucw_stack_off, &c->ucw_stack, &c->ucw_paths, &c->ucw_len, &c->ucw_scores, &c->ucw_n, &c->ucw_status, &c->ucw_thr, &c->ucw_plen, &c->ucw_pathbuf, &c->ucw_flags, &c->ucw_flag_off,
+                   &c->prof8, &c->prof8_off, &c->proff, &c->proff_off};
   for (DevBuf* d : all) d->release();
   if (c->pin) cudaFreeHost(c->pin);
   if (c->pin_flag) cudaFreeHost(c->pin_flag);
@@ -1184,6 +1232,7 @@ int aadp_set_scoring(aadp_ctx* c, const float* sub, int A, float gi, float ge, i
     for (int i = 0; i < A * A && ok; ++i) ok = (sub[i] * m == rintf(sub[i] * m));
     if (ok) s = t;
   }
+  c->prof_mode = false;
   c->sc.A = A;
   c->sc.delfree = (align_type == AADP_LOCAL || align_type == AADP_SEMI_LOCAL || align_type == AADP_LOCAL_GLOBAL);
   c->sc.insfree = (align_type == AADP_LOCAL || align_type == AADP_SEMI_LOCAL || align_type == AADP_GLOBAL_LOCAL);
@@ -1247,6 +1296,106 @@ int aadp_set_scoring(aadp_ctx* c, const float* sub, int A, float gi, float ge, i
     CK(cudaMemcpy(c->sub8p.p, pad.data(), pad.size(), cudaMemcpyHostToDevice));
   }
   CK(cudaStreamSynchronize(c->stream));
+  c->have_scoring = true;
+  return 0;
+}
+
+int aadp_set_profile_scoring(aadp_ctx* c, const float* prof, const int64_t* prof_off, int64_t nprof, int A, float gi,
+                             float ge, int align_type, uint32_t flags) {
+  if (check_ctx(c, false)) return 1;
+  if (A < 1 || A > 64) return fail("alphabet size must be 1..64");
+  if (align_type < 0 || align_type > 4) return fail("Illegal gap style");  // aasubalib.h:49
+  if (!(gi >= 0.f) || !(ge >= 0.f)) return fail("gap penalties must be non-negative");
+  if (nprof < 0 || nprof > 0x7fffffff || !prof_off) return fail("null input");
+  if (prof_off[nprof] > prof_off[0] && !prof) return fail("null input");
+  const char* other = "; position-specific similarities off that grid run on the exact fp32 kernels of aadp_fill_batch_tabulated / "
+                      "aadp_fill_pair_general";
+  if (c->force_float)
+    return fail(std::string("aadp_set_profile_scoring: profile scoring runs on the integer kernels only and the option exact_float "
+                            "is set") + other);
+  for (int64_t s2 = 0; s2 < nprof; ++s2) {
+    const int64_t n = prof_off[s2 + 1] - prof_off[s2];
+    if (n < 0) return fail("aadp_set_profile_scoring: profile offsets must be non-decreasing");
+    if (n % A) return fail("aadp_set_profile_scoring: the profile of sequence " + std::to_string(s2) + " has " + std::to_string(n) +
+                           " entries, not a multiple of A = " + std::to_string(A));
+  }
+  const float* p0 = prof ? prof + prof_off[0] : nullptr;
+  const int64_t ntot = prof_off[nprof] - prof_off[0];
+  // the dyadic grid of aadp_set_scoring: smallest s <= 8 with every entry, gi and ge integral in units of 2^-s
+  int s = -1;
+  for (int t = 0; t <= 8 && s < 0; ++t) {
+    const float m = (float)(1 << t);
+    bool ok = (gi * m == rintf(gi * m)) && (ge * m == rintf(ge * m));
+    for (int64_t i = 0; i < ntot && ok; ++i) ok = (p0[i] * m == rintf(p0[i] * m));
+    if (ok) s = t;
+  }
+  if (s < 0) return fail(std::string("aadp_set_profile_scoring: the profile entries, gi and ge are not on one dyadic grid 2^-s, s <= 8") + other);
+  const float m = (float)(1 << s);
+  if (gi * m > 1e6f || ge * m > 1e5f) return fail(std::string("aadp_set_profile_scoring: gap penalties too large for the integer kernels") + other);
+  std::vector<int> pmax((size_t)nprof, 0);
+  for (int64_t s2 = 0; s2 < nprof; ++s2)
+    for (int64_t i = prof_off[s2]; i < prof_off[s2 + 1]; ++i) {
+      const float v = fabsf(prof[i] * m);
+      if (v > 127.f) {
+        char e[256];
+        snprintf(e, sizeof e, "aadp_set_profile_scoring: the profile of sequence %lld has an entry of %g = %g units of 2^-%d, above 127 units",
+                 (long long)s2, (double)prof[i], (double)v, s);
+        return fail(e + std::string(other));
+      }
+      pmax[(size_t)s2] = std::max(pmax[(size_t)s2], (int)v);
+    }
+  // int8 layout (ProfDev, aadp_kernels.cuh): per sequence, forward flow then reverse flow, A rows of prof_row_bytes(L)
+  std::vector<int64_t> off8((size_t)nprof + 1, 0), offf((size_t)nprof + 1, 0);
+  for (int64_t s2 = 0; s2 < nprof; ++s2) {
+    const int L = (int)((prof_off[s2 + 1] - prof_off[s2]) / A);
+    off8[(size_t)s2 + 1] = off8[(size_t)s2] + 2 * (int64_t)A * prof_row_bytes(L);
+    offf[(size_t)s2 + 1] = prof_off[s2 + 1] - prof_off[0];
+  }
+  std::vector<int8_t> p8((size_t)std::max<int64_t>(off8[(size_t)nprof], 16), (int8_t)-128);
+  for (int64_t s2 = 0; s2 < nprof; ++s2) {
+    const float* ps = prof + prof_off[s2];
+    const int L = (int)((prof_off[s2 + 1] - prof_off[s2]) / A), nb = prof_row_bytes(L), sig = nb - L;
+    int8_t* fwd = p8.data() + off8[(size_t)s2];
+    int8_t* rev = fwd + (int64_t)A * nb;
+    for (int j = 1; j <= L; ++j)
+      for (int a = 0; a < A; ++a) {
+        const int8_t v = (int8_t)(int)(ps[(int64_t)(j - 1) * A + a] * m);
+        fwd[(int64_t)a * nb + j - 1 + sig] = v;  // forward flow column j
+        rev[(int64_t)a * nb + L - j] = v;        // reverse flow column L+1-j
+      }
+  }
+  // everything checked: the profiles replace the context's scoring
+  CK(cudaStreamSynchronize(c->stream));
+  if (c->prof8.reserve(p8.size()) || c->prof8_off.reserve(off8.size() * 8) || c->proff.reserve(std::max<size_t>((size_t)ntot * 4, 16)) ||
+      c->proff_off.reserve(offf.size() * 8))
+    return 1;
+  CK(cudaMemcpy(c->prof8.p, p8.data(), p8.size(), cudaMemcpyHostToDevice));
+  CK(cudaMemcpy(c->prof8_off.p, off8.data(), off8.size() * 8, cudaMemcpyHostToDevice));
+  if (ntot) CK(cudaMemcpy(c->proff.p, p0, (size_t)ntot * 4, cudaMemcpyHostToDevice));
+  CK(cudaMemcpy(c->proff_off.p, offf.data(), offf.size() * 8, cudaMemcpyHostToDevice));
+  c->proff_h.assign(p0, p0 + ntot);
+  c->proff_off_h = offf;
+  c->prof_len.resize((size_t)nprof);
+  for (int64_t s2 = 0; s2 < nprof; ++s2) c->prof_len[(size_t)s2] = prof_off[s2 + 1] - prof_off[s2];
+  c->prof_max = pmax;
+  c->prof_nseq = nprof;
+  c->prof_mode = true;
+  c->float_mode = false;
+  c->max_abs_sub = 0;
+  c->sc.A = A;
+  c->sc.gi = (int)(gi * m);
+  c->sc.ge = (int)(ge * m);
+  c->sc.delfree = (align_type == AADP_LOCAL || align_type == AADP_SEMI_LOCAL || align_type == AADP_LOCAL_GLOBAL);
+  c->sc.insfree = (align_type == AADP_LOCAL || align_type == AADP_SEMI_LOCAL || align_type == AADP_GLOBAL_LOCAL);
+  c->sc.local = (align_type == AADP_LOCAL);
+  c->sc.scale_log2 = s;
+  c->align_type = align_type;
+  c->flags = flags;
+  c->gi_f = gi;
+  c->ge_f = ge;
+  c->b.ran_what = 0;
+  c->b.sched_ok = false;  // as aadp_set_scoring: classification, bounds and storage modes depend on the scoring
+  if (c->b.seq_A != A) c->b.have_seqs = false;
   c->have_scoring = true;
   return 0;
 }
@@ -1456,18 +1605,28 @@ int aadp_cross_run(aadp_ctx* c, const int32_t* q_ids, int64_t nq, const int32_t*
   auto len = [&](int32_t s2) { return b.seq_off[(size_t)s2 + 1] - b.seq_off[(size_t)s2]; };
   for (int64_t i = 0; i < nq; ++i) if (q_ids[i] < 0 || q_ids[i] >= b.nseq) return fail("query id out of range");
   for (int64_t i = 0; i < nt; ++i) if (t_ids[i] < 0 || t_ids[i] >= b.nseq) return fail("template id out of range");
+  if (c->prof_mode) {
+    if (profile_count_refusal(c, b.nseq)) return 1;
+    for (int64_t i = 0; i < nt; ++i)
+      if (c->prof_len[(size_t)t_ids[i]] != len(t_ids[i]) * c->sc.A) return profile_refusal(c, t_ids[i], len(t_ids[i]));
+  }
   // ---- which templates / queries qualify for the packed int16x2 kernel (same rules as build_batch_meta)
   const bool packed_mode = c->allow_packed && !c->float_mode && !c->sc.local && c->sc.ge <= 400 && c->sc.gi <= 2048;
   std::vector<int32_t> te, qe, tbad, qbad;  // LIST indices
   int64_t maxLt = 0;
+  int64_t mx = c->max_abs_sub;  // |similarity| bound; profile scoring: the largest of the packed templates of this call
   for (int64_t i = 0; i < nt; ++i) {
     const int64_t L = len(t_ids[i]);
-    if (packed_mode && L >= 1 && L <= 512) { te.push_back((int32_t)i); maxLt = std::max(maxLt, L); }
+    if (packed_mode && L >= 1 && L <= 512) {
+      te.push_back((int32_t)i);
+      maxLt = std::max(maxLt, L);
+      if (c->prof_mode) mx = std::max<int64_t>(mx, c->prof_max[(size_t)t_ids[i]]);
+    }
     else tbad.push_back((int32_t)i);
   }
   for (int64_t i = 0; i < nq; ++i) {
     const int64_t L = len(q_ids[i]);
-    const int64_t bd = std::min(L, maxLt) * (int64_t)c->max_abs_sub + 2 * (int64_t)c->sc.gi + (int64_t)c->sc.ge * (L + maxLt);
+    const int64_t bd = std::min(L, maxLt) * mx + 2 * (int64_t)c->sc.gi + (int64_t)c->sc.ge * (L + maxLt);
     if (!te.empty() && L >= 1 && bd < kPackedBound) qe.push_back((int32_t)i);
     else qbad.push_back((int32_t)i);
   }
@@ -1501,7 +1660,8 @@ int aadp_cross_run(aadp_ctx* c, const int32_t* q_ids, int64_t nq, const int32_t*
     std::vector<int32_t> qid(q_ids, q_ids + nq), tid(t_ids, t_ids + nt);
     if (upload_vec(c, c->x_layout, layouts) || upload_vec(c, c->x_qc, qc) || upload_vec(c, c->x_qid, qid) ||
         upload_vec(c, c->x_tid, tid)) return 1;
-    auto kern = packed_kernel<0, 0, 0, 1>;
+    const bool pro = c->prof_mode;
+    const void* kern = pro ? (const void*)packed_kernel<0, 0, 0, 1, 0, 1> : (const void*)packed_kernel<0, 0, 0, 1, 0, 0>;
     const int A = c->sc.A;
     const size_t smem = packed_smem_bytes(A, 0, 1);
     CK(cached_max_smem((const void*)kern, (size_t)(smem)));
@@ -1540,8 +1700,10 @@ int aadp_cross_run(aadp_ctx* c, const int32_t* q_ids, int64_t nq, const int32_t*
     Q.cells_hint = sq * st;
     c->x_cells += sq * st;
     const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(resident, Q.n_tasks));
-    c->prof_begin("packed_kernel<TB=0,FST=0,MSK=0,XM=1>fwd", Q.cells_hint);
-    kern<<<grid, kPackedWarps * 32, smem, c->stream>>>(Q);
+    c->prof_begin(pro ? "packed_kernel<TB=0,FST=0,MSK=0,XM=1,PRO=1>fwd" : "packed_kernel<TB=0,FST=0,MSK=0,XM=1>fwd", Q.cells_hint);
+    Q.prof = c->prof_dev();
+    if (pro) packed_kernel<0, 0, 0, 1, 0, 1><<<grid, kPackedWarps * 32, smem, c->stream>>>(Q);
+    else packed_kernel<0, 0, 0, 1, 0, 0><<<grid, kPackedWarps * 32, smem, c->stream>>>(Q);
     c->prof_end();
     CK(cudaGetLastError());
     c->launches++;
@@ -1958,8 +2120,9 @@ static int run_batch_impl(aadp_ctx* c, uint32_t what, float delta_ratio, float* 
     M.threshold = d_threshold;
     M.count = reinterpret_cast<long long*>(d_nearopt_count);
     if (!b.order[0].empty() || !b.order[1].empty()) {
-      c->prof_begin("mask_kernel", 0);
-      mask_kernel<<<(int)np, 256, 0, c->stream>>>(M);
+      c->prof_begin(c->prof_mode ? "mask_kernel<PRO=1>" : "mask_kernel", 0);
+      if (c->prof_mode) mask_kernel<1><<<(int)np, 256, 0, c->stream>>>(M, c->prof_dev());
+      else mask_kernel<0><<<(int)np, 256, 0, c->stream>>>(M, c->prof_dev());
       c->prof_end();
       CK(cudaGetLastError());
       c->launches++;
@@ -1968,8 +2131,9 @@ static int run_batch_impl(aadp_ctx* c, uint32_t what, float delta_ratio, float* 
       M.want_fmt = 2;
       M.only_pair = p;
       if (d_nearopt_count) CK(cudaMemsetAsync(d_nearopt_count + p, 0, 8, c->stream));
-      c->prof_begin("mask_kernel(long pair)", 0);
-      mask_kernel<<<dim3(1, 2368), 256, 0, c->stream>>>(M);
+      c->prof_begin(c->prof_mode ? "mask_kernel<PRO=1>(long pair)" : "mask_kernel(long pair)", 0);
+      if (c->prof_mode) mask_kernel<1><<<dim3(1, 2368), 256, 0, c->stream>>>(M, c->prof_dev());
+      else mask_kernel<0><<<dim3(1, 2368), 256, 0, c->stream>>>(M, c->prof_dev());
       c->prof_end();
       CK(cudaGetLastError());
       c->launches++;
@@ -2191,6 +2355,9 @@ int aadp_fill_pair(aadp_ctx* c, const uint8_t* q, int Lq, const uint8_t* t, int 
                    float* score_fwd, int32_t* prevq_fwd, int32_t* prevt_fwd, float* score_rev, int32_t* prevq_rev,
                    int32_t* prevt_rev, uint8_t* nearopt, float* threshold) {
   if (check_ctx(c, true)) return 1;
+  if (c->prof_mode)
+    return fail("aadp_fill_pair: profile scoring selects the similarity by template sequence id, which a single pair does not "
+                "have; use a one-pair batch (aadp_fill_batch + aadp_batch_fetch_pair)");
   if (Lq < 0 || Lt < 0) return fail("Illegal bounds building DPM");  // dpmatrix.h:360-361
   if (direction < 1 || direction > 3) return fail("bad direction");
   std::vector<uint8_t> res((size_t)Lq + Lt + 1);
@@ -2688,9 +2855,16 @@ static int near_optimal_impl(aadp_ctx* c, int cno, const uint8_t* flags, const i
   U.stack = c->ucw_stack.as<int4>();
   c->launches = 0;
   if (!c->float_mode) {
-    c->prof_begin(cno ? "ucw_enum_kernel<CNO=1>" : "ucw_enum_kernel<CNO=0>", 0);
-    if (cno) ucw_enum_kernel<1><<<(unsigned)((n * 32 + 127) / 128), 128, 0, c->stream>>>(U);
-    else ucw_enum_kernel<0><<<(unsigned)((n * 32 + 127) / 128), 128, 0, c->stream>>>(U);
+    const unsigned grid = (unsigned)((n * 32 + 127) / 128);
+    if (c->prof_mode) {
+      c->prof_begin(cno ? "ucw_enum_kernel<CNO=1,PRO=1>" : "ucw_enum_kernel<CNO=0,PRO=1>", 0);
+      if (cno) ucw_enum_kernel<1, 1><<<grid, 128, 0, c->stream>>>(U, c->prof_dev());
+      else ucw_enum_kernel<0, 1><<<grid, 128, 0, c->stream>>>(U, c->prof_dev());
+    } else {
+      c->prof_begin(cno ? "ucw_enum_kernel<CNO=1>" : "ucw_enum_kernel<CNO=0>", 0);
+      if (cno) ucw_enum_kernel<1, 0><<<grid, 128, 0, c->stream>>>(U, c->prof_dev());
+      else ucw_enum_kernel<0, 0><<<grid, 128, 0, c->stream>>>(U, c->prof_dev());
+    }
     c->prof_end();
     CK(cudaGetLastError());
     c->launches++;
@@ -2727,8 +2901,8 @@ static int near_optimal_impl(aadp_ctx* c, int cno, const uint8_t* flags, const i
       V.threshold = U.threshold + k0;
       if (flags) V.subopt_off = U.subopt_off + k0;
       c->prof_begin("ucw_enum_kernel (exact float)", 0);
-      if (cno) ucw_enum_kernel<1><<<(unsigned)((m * 32 + 127) / 128), 128, 0, c->stream>>>(V);
-      else ucw_enum_kernel<0><<<(unsigned)((m * 32 + 127) / 128), 128, 0, c->stream>>>(V);
+      if (cno) ucw_enum_kernel<1, 0><<<(unsigned)((m * 32 + 127) / 128), 128, 0, c->stream>>>(V, c->prof_dev());
+      else ucw_enum_kernel<0, 0><<<(unsigned)((m * 32 + 127) / 128), 128, 0, c->stream>>>(V, c->prof_dev());
       c->prof_end();
       CK(cudaGetLastError());
       c->launches++;
@@ -2800,7 +2974,9 @@ int aadp_batch_near_optimal_pruned(aadp_ctx* c, int64_t pair_id, int variant, co
   CK(cudaStreamSynchronize(c->stream));
   const int A = c->sc.A;
   for (int i = 1; i <= Lq; ++i)
-    for (int j = 1; j <= Lt; ++j) sim[(size_t)i * (Lt + 2) + j] = c->subf_h[(size_t)qr[(size_t)i - 1] * A + tr[(size_t)j - 1]];
+    for (int j = 1; j <= Lt; ++j)
+      sim[(size_t)i * (Lt + 2) + j] = c->prof_mode ? c->proff_h[(size_t)(c->proff_off_h[(size_t)ts] + (int64_t)(j - 1) * A + qr[(size_t)i - 1])]
+                                                   : c->subf_h[(size_t)qr[(size_t)i - 1] * A + tr[(size_t)j - 1]];
   PrunedParams Q;
   Q.Lq = Lq; Q.Lt = Lt;
   Q.F = F.data(); Q.pq = pq.data(); Q.pt = pt.data(); Q.sim = sim.data();
@@ -2845,6 +3021,9 @@ int aadp_batch_near_optimal_constrained(aadp_ctx* c, const int64_t* pair_ids, in
 int aadp_fill_subpair(aadp_ctx* c, const uint8_t* q, int Lq, const uint8_t* t, int Lt, int q1_end, int t1_end, int q2_beg,
                       int t2_beg, int direction, float* score, int32_t* prev_q, int32_t* prev_t) {
   if (check_ctx(c, true)) return 1;
+  if (c->prof_mode)
+    return fail("aadp_fill_subpair: sub-rectangle fills run on the exact fp32 kernels, which profile scoring does not drive; use "
+                "aadp_fill_pair_general with a rectangle and the profile's similarity matrix");
   if (Lq < 0 || Lt < 0) return fail("Illegal bounds building DPM");
   if (direction != AADP_FWD && direction != AADP_REV) return fail("bad direction");
   // dpmatrix.h:360-361 (and the matrix limits the reference does not check)
@@ -2874,6 +3053,9 @@ int aadp_fill_subpair_batch(aadp_ctx* c, const uint8_t* residues, const int64_t*
                             const int32_t* item_t, const int32_t* rects, int64_t nitems, int direction, float* score,
                             int64_t* ali_off, int32_t* pairs, int64_t pairs_cap, int32_t* n_out, int32_t* status) {
   if (check_ctx(c, true)) return 1;
+  if (c->prof_mode)
+    return fail("aadp_fill_subpair_batch: sub-rectangle fills run on the exact fp32 kernels, which profile scoring does not drive; "
+                "use aadp_fill_pair_general with a rectangle and the profile's similarity matrix");
   if (direction != AADP_FWD && direction != AADP_REV) return fail("bad direction");
   if (nitems < 0 || nitems > 0x7fffffff) return fail("bad batch size");
   if (nitems && (!item_q || !item_t || !rects || !seq_off)) return fail("null input");

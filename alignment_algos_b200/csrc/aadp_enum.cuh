@@ -82,8 +82,9 @@ struct UcwParams {
   int2* pathbuf;              // the partial alignment from the final cell down to the current node
 };
 
-template <int CNO>
-__global__ void __launch_bounds__(128, 8) ucw_enum_kernel(const UcwParams P) {
+// PRO = 1: sim() reads the fp32 position-specific template profile (ProfDev, aadp_set_profile_scoring); exact on the grid.
+template <int CNO, int PRO = 0>
+__global__ void __launch_bounds__(128, 8) ucw_enum_kernel(const UcwParams P, const ProfDev pd) {
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (warp >= P.n) return;
   const int64_t pair = P.ids[warp];
@@ -115,6 +116,7 @@ __global__ void __launch_bounds__(128, 8) ucw_enum_kernel(const UcwParams P) {
   };
   auto sim = [&](int i, int j) -> float {  // aasubalib.h:17-25
     if (i < 1 || i > Lq || j < 1 || j > Lt) return 0.f;
+    if constexpr (PRO) return pd.pf[pd.offf[ts] + (int64_t)(j - 1) * P.A + (int)qseq[i - 1]];
     return P.subf[(int)qseq[i - 1] * P.A + (int)tseq[j - 1]];
   };
   auto pen = [&](int len) { return __fadd_rn(P.gi, __fmul_rn(P.ge, (float)(len - 1))); };

@@ -91,6 +91,25 @@ struct FillParams {
   long long* wave_dbg;       // optional [stripe][2]: cycles spent waiting for the left neighbour, total cycles
 };
 
+// Position-specific template profiles (aadp_set_profile_scoring): sim(i,j) = profile of the template at position j,
+// query code q_i.  The int8 copy (grid units) is laid out per sequence and FLOW: sequence s owns 2*A*16n bytes at
+// p8 + off8[s] (n = ceil(L/16)), the forward flow first, then the reverse flow.  Row a of a flow holds 16n bytes; byte k
+// is the score of query code a at flow column j = k + 1 - sig, -128 where that column does not exist.  Forward: sig =
+// 16n - L (right-aligned like the packed forward pass); reverse: sig = 0 and flow column j is template position L+1-j.
+// A packed lane therefore loads its 16 columns of a row with one aligned 16-byte load.  pf / offf: the profiles as
+// given (fp32, [offf[s] + (j-1)*A + a]) for the enumeration kernel.
+struct ProfDev {
+  const int8_t* p8;
+  const int64_t* off8;
+  const float* pf;
+  const int64_t* offf;
+};
+__host__ __device__ inline int prof_row_bytes(int L) { return 16 * ((L + 15) >> 4); }
+// row 0 of the flow `rev` of sequence s (template length L)
+__device__ __forceinline__ const int8_t* prof_flow(const ProfDev& pd, int s, int L, int A, int rev) {
+  return pd.p8 + pd.off8[s] + (rev ? (int64_t)A * prof_row_bytes(L) : 0);
+}
+
 __device__ __forceinline__ int ld_acquire(const int* p) {
   int v;
   asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
@@ -134,9 +153,12 @@ __device__ __forceinline__ int sext8(uint32_t w, int c) {
 // WAVE = 1: this warp (one CTA) fills ONLY stripe `wave_st` of the pair; stripe st consumes the boundary
 // column of stripe st-1 from global memory 32 rows at a time, gated by release/acquire progress flags --
 // the CTAs of one launch form an anti-diagonal wavefront over the column stripes of one long pair.
-template <int K, int TBM, int STM, int WAVE>
+// PRO = 1: the stripe profile is copied from the template's position-specific profile (ProfDev) instead of being
+// built from the substitution table; nothing else changes.
+template <int K, int TBM, int STM, int WAVE, int PRO = 0>
 __device__ __forceinline__ void fill_pair_warp(const FillParams& P, int pair, int8_t* prof, uint8_t* qring,
-                                               const int8_t* s_sub, int4* bb, int lane, int wave_st = 0) {
+                                               const int8_t* s_sub, int4* bb, int lane, int wave_st = 0,
+                                               const ProfDev& pd = ProfDev{}) {
   constexpr int W = 32 * K;
   const Scoring& S = P.sc;
   const int gi = S.gi, ge = S.ge;
@@ -183,7 +205,26 @@ __device__ __forceinline__ void fill_pair_warp(const FillParams& P, int pair, in
     const int n_act = (cols_here + K - 1) / K;
 
     // ---- template profile for this stripe: prof[a*W + lane*K + c] = sub8[a][t_(jbase+c+1)]
-    {
+    if (PRO) {
+      // flow column j of the stripe sits at byte j-1+sig of the row; columns beyond Lt are never read back
+      const int nb = prof_row_bytes(Lt), sig = rev ? 0 : nb - Lt;
+      const int8_t* src = prof_flow(pd, ts, Lt, S.A, rev) + sig - 1;
+      __syncwarp();  // previous users of prof are done
+      for (int a = 0; a < S.A; ++a) {
+        uint32_t* dst = reinterpret_cast<uint32_t*>(prof + a * W + lane * K);
+#pragma unroll
+        for (int w = 0; w < K / 4; ++w) {
+          uint32_t o = 0;
+#pragma unroll
+          for (int b = 0; b < 4; ++b) {
+            const int j = jbase + w * 4 + b + 1;
+            if (j <= Lt) o |= (uint32_t)(uint8_t)src[a * nb + j] << (8 * b);
+          }
+          dst[w] = o;
+        }
+      }
+      __syncwarp();
+    } else {
       uint32_t tc[K / 4];
 #pragma unroll
       for (int w = 0; w < K / 4; ++w) {
@@ -463,8 +504,9 @@ __device__ __forceinline__ void fill_pair_warp(const FillParams& P, int pair, in
   }
 }
 
-template <int K, int TBM, int STM>
-__global__ void __launch_bounds__(kWarpsPerCta * 32) fill_kernel(const FillParams P) {
+// PRO = 1: position-specific template profiles (aadp_set_profile_scoring, read from pd); PRO = 0 ignores pd
+template <int K, int TBM, int STM, int PRO>
+__global__ void __launch_bounds__(kWarpsPerCta * 32) fill_kernel(const FillParams P, const ProfDev pd) {
   extern __shared__ __align__(16) unsigned char smem[];
   constexpr int W = 32 * K;
   const int A = P.sc.A;
@@ -473,7 +515,8 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) fill_kernel(const FillParam
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   uint8_t* qring = smem + sub_bytes + warp * kQRing;
   int8_t* prof = reinterpret_cast<int8_t*>(smem + sub_bytes + kWarpsPerCta * kQRing + warp * A * W);
-  for (int x = threadIdx.x; x < A * A; x += blockDim.x) s_sub[x] = P.sub8[x];
+  if (!PRO)
+    for (int x = threadIdx.x; x < A * A; x += blockDim.x) s_sub[x] = P.sub8[x];
   __syncthreads();
   const int slot = blockIdx.x * kWarpsPerCta + warp;
   int4* bb = P.bbuf ? P.bbuf + (int64_t)slot * P.bb_rows : nullptr;
@@ -482,14 +525,14 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) fill_kernel(const FillParam
     if (lane == 0) item = atomicAdd(P.counter, 1u);
     item = __shfl_sync(0xffffffffu, item, 0);
     if (item >= (unsigned int)P.n_items) break;
-    fill_pair_warp<K, TBM, STM, 0>(P, P.order[item], prof, qring, s_sub, bb, lane);
+    fill_pair_warp<K, TBM, STM, 0, PRO>(P, P.order[item], prof, qring, s_sub, bb, lane, 0, pd);
   }
 }
 
 // One long pair, both directions in one launch: CTA b (one warp) fills stripe b % nstripes of direction
 // b / nstripes.  All CTAs must be co-resident (they wait on each other): launched cooperatively.
-template <int K, int TBM, int STM>
-__global__ void __launch_bounds__(32) wave_kernel(const FillParams Pf, const FillParams Pr, int ndirs) {
+template <int K, int TBM, int STM, int PRO>
+__global__ void __launch_bounds__(32) wave_kernel(const FillParams Pf, const FillParams Pr, int ndirs, const ProfDev pd) {
   extern __shared__ __align__(16) unsigned char smem[];
   constexpr int W = 32 * K;
   const int nst = Pf.wave_nstripes;
@@ -502,10 +545,12 @@ __global__ void __launch_bounds__(32) wave_kernel(const FillParams Pf, const Fil
   const int lane = threadIdx.x;
   uint8_t* qring = smem + sub_bytes;  // followed by the 512-byte staging block of the input boundary
   int8_t* prof = reinterpret_cast<int8_t*>(smem + sub_bytes + kQRing + 512);
-  for (int x = threadIdx.x; x < A * A; x += blockDim.x) s_sub[x] = P.sub8[x];
+  if (!PRO)
+    for (int x = threadIdx.x; x < A * A; x += blockDim.x) s_sub[x] = P.sub8[x];
   __syncwarp();
-  fill_pair_warp<K, TBM, STM, 1>(P, P.wave_pair, prof, qring, s_sub, nullptr, lane, st);
+  fill_pair_warp<K, TBM, STM, 1, PRO>(P, P.wave_pair, prof, qring, s_sub, nullptr, lane, st, pd);
 }
+
 
 // ------------------------------------------------------------------------------------------------
 // Packed-traceback decode (shared by host and device).
@@ -640,7 +685,8 @@ __device__ __forceinline__ float nearopt_threshold(float opt, float delta_ratio)
 #define AADP_MASK_U 4
 #endif
 constexpr int kMaskU = AADP_MASK_U;  // 32-column groups a warp loads before it uses any (bytes in flight per thread)
-__global__ void __launch_bounds__(256) mask_kernel(const MaskParams P) {
+template <int PRO>
+__global__ void __launch_bounds__(256) mask_kernel(const MaskParams P, const ProfDev pd) {
   const int pair = P.only_pair >= 0 ? P.only_pair : blockIdx.x;
   if (P.fmt[pair] != P.want_fmt) return;
   const int qs = P.pair_q[pair], ts = P.pair_t[pair];
@@ -665,9 +711,11 @@ __global__ void __launch_bounds__(256) mask_kernel(const MaskParams P) {
   // reference's float comparison equals  slack > floor(thr * 2^s)  on the integers (the packed kernels use the same form).
   const int thr_i = (int)fminf(fmaxf(floorf(thr * (float)(1 << P.sc.scale_log2)), -2.0e9f), 2.0e9f);
   const uint8_t* tres = P.residues + to;
+  // PRO: the forward-flow profile row of the query code, shifted so that column jm+1 is subrow[jm]
+  const int8_t* prof0 = PRO ? prof_flow(pd, ts, Lt, A, 0) + (prof_row_bytes(Lt) - Lt) : nullptr;
   for (int i = i_lo; i <= i_hi; ++i) {
     const int qa = P.residues[qo + i - 1];
-    const int8_t* subrow = P.sub8 + qa * A;
+    const int8_t* subrow = PRO ? prof0 + qa * prof_row_bytes(Lt) : P.sub8 + qa * A;
     // row pointers: forward row i ascending, reverse row Lq-i descending (the reverse matrix is stored in flow coordinates)
     const int16_t* f16 = (const int16_t*)P.scF + so + (int64_t)(i - 1) * scs;
     const int16_t* r16 = (const int16_t*)P.scR + so + (int64_t)(Lq - i) * scs + (Lt - 1);
@@ -685,7 +733,7 @@ __global__ void __launch_bounds__(256) mask_kernel(const MaskParams P) {
           int f, r;
           if (P.st_mode == 1) { f = f16[jm]; r = r16[-jm]; }
           else { f = f32[jm]; r = r32[-jm]; }
-          on[u] = f + r - (int)subrow[tres[jm]] > thr_i;
+          on[u] = f + r - (int)subrow[PRO ? jm : tres[jm]] > thr_i;
         }
       }
       uint32_t mine = 0;

@@ -114,6 +114,7 @@ struct PackedParams {
   int x_nlayouts, x_nqc, x_group;
   long long x_nt;            // row stride of x_scores
   float* x_scores;           // [query list index][template list index] = D[last][last].score
+  ProfDev prof;              // position-specific template profiles (read by the PRO = 1 kernels only)
 };
 
 __device__ __forceinline__ uint32_t pk2(int lo, int hi) { return ((uint32_t)lo & 0xffffu) | ((uint32_t)hi << 16); }
@@ -234,7 +235,9 @@ struct RowSum {
 // (s = max(0.f, s), :580 etc.), i.e. M = max(0, sim + X); the gap states stay unclamped (they only ever lose against
 // M >= 0 where the clamp would have mattered), a cell clamped to 0 keeps its match predecessor (decoded from the
 // stored score, dense_kernel / local_traceback_kernel).  One more VIMNMX per packed cell.
-template <int TBM, int FST, int MSK, int XM, int LOC = 0>
+// PRO = 1: position-specific template profiles (ProfDev, aadp_set_profile_scoring): the profile rows are copied from the
+// template's int8 profile of this flow instead of being built from the substitution table; the row loop is unchanged.
+template <int TBM, int FST, int MSK, int XM, int LOC = 0, int PRO = 0>
 __device__ __forceinline__ void packed_task(const PackedParams& P, int task, int8_t* prof, int4* red,
                                             uint8_t* stage, int lane) {
   const Scoring& S = P.sc;
@@ -284,7 +287,24 @@ __device__ __forceinline__ void packed_task(const PackedParams& P, int task, int
 
   // ---- template profiles: prof[a*512 + lane*16 + c] = sub8[a][t_(column of register c)], pads = -128
   // (cross mode: one profile for both halves, built once per item and reused by every query couple)
-  if (!XM || rep == 0) {
+  if constexpr (PRO) {
+    if (!XM || rep == 0) {
+      // lane `off` of a segment owns bytes 16*off .. 16*off+15 of every profile row of the flow: one aligned 16-byte load
+      // per row; the -128 pad columns are already in place.  A half without a pair gets pad columns only.
+      __syncwarp();
+#pragma unroll
+      for (int h = 0; h < (XM ? 1 : 2); ++h) {
+        const int ts = pid[h] < 0 ? -1 : (XM ? P.x_tid[pid[h]] : P.pair_t[pid[h]]);
+        const int nb = prof_row_bytes(Lt[h]);
+        const int8_t* src = ts < 0 ? nullptr : prof_flow(P.prof, ts, Lt[h], A, P.rev) + off * 16;
+        int8_t* dst = (h ? profB : profA) + lane * 16;
+        for (int a = 0; a < A; ++a)
+          *reinterpret_cast<uint4*>(dst + a * W) = ts < 0 ? make_uint4(0x80808080u, 0x80808080u, 0x80808080u, 0x80808080u)
+                                                          : *reinterpret_cast<const uint4*>(src + a * nb);
+      }
+      __syncwarp();
+    }
+  } else if (!XM || rep == 0) {
     // padded substitution table (A rows of A+1 entries, entry A = pad = -128) into the staging area: no cp.async
     // of this task has been issued yet and the previous task drained its own
     int8_t* s_sub = reinterpret_cast<int8_t*>(stage);
@@ -752,7 +772,7 @@ __device__ __forceinline__ void packed_task(const PackedParams& P, int task, int
   }  // rep
 }
 
-template <int TBM, int FST, int MSK, int XM, int LOC = 0>
+template <int TBM, int FST, int MSK, int XM, int LOC = 0, int PRO = 0>
 __global__ void __launch_bounds__(kPackedWarps * 32) __maxnreg__(XM ? 168 : (MSK ? 255 : (TBM ? 224 : 200))) packed_kernel(const PackedParams P) {
   extern __shared__ __align__(16) unsigned char smem[];
   const int A = P.sc.A;
@@ -772,7 +792,7 @@ __global__ void __launch_bounds__(kPackedWarps * 32) __maxnreg__(XM ? 168 : (MSK
     if (lane == 0) item = atomicAdd(P.counter, 1u);
     item = __shfl_sync(0xffffffffu, item, 0);
     if (item >= (unsigned int)P.n_tasks) break;
-    packed_task<TBM, FST, MSK, XM, LOC>(P, (int)item, prof, red, stage, lane);
+    packed_task<TBM, FST, MSK, XM, LOC, PRO>(P, (int)item, prof, red, stage, lane);
   }
 }
 

@@ -97,6 +97,26 @@ int aadp_set_option(aadp_ctx* ctx, const char* key, int value);
 int aadp_set_scoring(aadp_ctx* ctx, const float* sub, int A, float gi, float ge, int align_type,
                      uint32_t flags);
 
+/* ---- scoring by POSITION-SPECIFIC TEMPLATE PROFILES (a PSSM per template) on the integer kernels: replaces the context's
+ * scoring like aadp_set_scoring (a later aadp_set_scoring switches back; both drop the resident batch's schedule).
+ * Profile s is prof[prof_off[s] .. prof_off[s+1]): L_s x A floats, row-major, row j-1 = the scores of query codes 0..A-1
+ * against template position j.  In every following batch or cross call a pair with template sequence id t uses
+ *     sim(i, j) = prof[prof_off[t] + (j-1)*A + q_i]        (border cells keep similarity 0)
+ * with gap(len) = gi + ge*(len-1) and the free end gaps of align_type, as aadp_set_scoring.  Queries are residue codes,
+ * validated against A as before; a sequence that is only ever a query may have an empty profile.
+ * Grid rule: every entry, gi and ge on one dyadic grid 2^-s, s <= 8, and |entry| <= 127 units of it -- anything else is
+ * refused (position-specific similarities off that grid: aadp_fill_batch_tabulated / aadp_fill_pair_general), and so is
+ * profile scoring while the option exact_float is set.  The packed-kernel bound and the int16/int32 score storage use
+ * each template's own max |entry| (cross calls: the largest over the packed templates of the call).
+ * Refused at run time, naming the sequence id: fewer than nseq profiles, a template whose profile is empty, a profile
+ * whose length is not L_t*A.
+ * Supported: aadp_fill_batch[_submit/_wait], aadp_upload_batch / aadp_run_batch (every AADP_W_* combination),
+ * aadp_batch_fetch_pair / _fetch_tb / aadp_decode_cell, aadp_batch_optimal[_all[_compact]], aadp_cross_run / _scores,
+ * aadp_batch_near_optimal[_constrained], aadp_batch_near_optimal_pruned.  Refused: aadp_fill_pair (no template id: use a
+ * one-pair batch), aadp_fill_subpair[_batch] (exact fp32 kernels only).                                                  */
+int aadp_set_profile_scoring(aadp_ctx* ctx, const float* prof, const int64_t* prof_off, int64_t nprof, int A,
+                             float gi, float ge, int align_type, uint32_t flags);
+
 /* ---- single pair, dense reference-shaped outputs: replaces the DPMatrix constructor
  * (dpmatrix.h:147-165) + build() (dpmatrix.h:291-317).  direction: AADP_FWD, AADP_REV or 3.
  * Outputs (host pointers, any may be NULL), all (Lq+2)*(Lt+2):
