@@ -332,7 +332,9 @@ __global__ void arena_kernel(const uint8_t* __restrict__ res, const int64_t* __r
 
 template <int TBM, int FST, int MSK, int LOC = 0, int PRO = 0>
 int launch_packed_t(aadp_ctx* c, PackedParams& P) {
-  auto kern = packed_kernel<TBM, FST, MSK, 0, LOC, PRO>;
+  // the forward pass with score spill reads its final row back (RB); a reverse pass with scores keeps the capture, its
+  // column Lt sits in a register picked at run time
+  auto kern = (FST && !MSK && !P.rev) ? packed_kernel<TBM, FST, MSK, 0, LOC, PRO, FST && !MSK> : packed_kernel<TBM, FST, MSK, 0, LOC, PRO>;
   const int A = P.sc.A;
   size_t smem = packed_smem_bytes(A, MSK);
   // measurement aid: AADP_PACKED_SMEM_PAD="fwd,rev" extra bytes per CTA lower the resident warps per SM

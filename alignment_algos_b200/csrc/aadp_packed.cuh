@@ -197,6 +197,19 @@ template <bool SA> __device__ __forceinline__ void cpa8(const SPtr& d, const voi
 __device__ __forceinline__ void prefetch_l2(const void* gsrc, int cond) {
   asm volatile("{ .reg .pred q; setp.ne.s32 q, %1, 0; @q prefetch.global.L2 [%0]; }" :: "l"(gsrc), "r"(cond) : "memory");
 }
+// Predicated global stores: the per-half store blocks of a row step become straight-line code (no BSSY/BRA)
+__device__ __forceinline__ void stg16_if(void* p, uint32_t a, uint32_t b, uint32_t c, uint32_t d, bool cond) {
+  asm volatile("{ .reg .pred q; setp.ne.s32 q, %5, 0; @q st.global.v4.u32 [%0], {%1,%2,%3,%4}; }"
+               :: "l"(p), "r"(a), "r"(b), "r"(c), "r"(d), "r"((int)cond) : "memory");
+}
+__device__ __forceinline__ void stg8_if(void* p, uint32_t a, uint32_t b, bool cond) {
+  asm volatile("{ .reg .pred q; setp.ne.s32 q, %3, 0; @q st.global.v2.u32 [%0], {%1,%2}; }"
+               :: "l"(p), "r"(a), "r"(b), "r"((int)cond) : "memory");
+}
+__device__ __forceinline__ void stg2_if(void* p, uint32_t a, bool cond) {
+  asm volatile("{ .reg .pred q; setp.ne.s32 q, %2, 0; @q st.global.u16 [%0], %1; }"
+               :: "l"(p), "h"((unsigned short)a), "r"((int)cond) : "memory");
+}
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 template <int N>
@@ -237,7 +250,9 @@ struct RowSum {
 // stored score, dense_kernel / local_traceback_kernel).  One more VIMNMX per packed cell.
 // PRO = 1: position-specific template profiles (ProfDev, aadp_set_profile_scoring): the profile rows are copied from the
 // template's int8 profile of this flow instead of being built from the substitution table; the row loop is unchanged.
-template <int TBM, int FST, int MSK, int XM, int LOC = 0, int PRO = 0>
+// RB = 1 (forward pass with score spill, FST = 1): the final-row summary reads M(Lq, .) back from the score blob instead
+// of parking the row state in local memory inside the row loop (see the capture below).
+template <int TBM, int FST, int MSK, int XM, int LOC = 0, int PRO = 0, int RB = 0>
 __device__ __forceinline__ void packed_task(const PackedParams& P, int task, int8_t* prof, int4* red,
                                             uint8_t* stage, int lane) {
   const Scoring& S = P.sc;
@@ -471,8 +486,15 @@ __device__ __forceinline__ void packed_task(const PackedParams& P, int task, int
     }
   }
   cp_async_commit();
-  int qa_n0 = 0, qa_n1 = 0;  // query residues of the NEXT row (read one row ahead to shorten the LDS chain)
+  // Row 1 of every lane: its residues and profile words are read here, before the loop, instead of behind an i == 1
+  // test in every step.  Waiting for the first group costs nothing extra: lane 0 of the warp waits for it in step 0.
+  cp_async_wait_all();
+  int qa_n0 = ld1<SA>(qst[0]), qa_n1 = ld1<SA>(qst[1]);  // query residues of the NEXT row (read one row ahead)
   uint4 pnA = make_uint4(0, 0, 0, 0), pnB = make_uint4(0, 0, 0, 0);  // profile words of the next row
+#if AADP_PROF_AHEAD
+  pnA = ld16<SA>(profA_s + qa_n0 * W);
+  pnB = ld16<SA>(profB_s + qa_n1 * W);
+#endif
   // valid (non-pad) registers in the layout of accM: A bytes 0/1 (even/odd c), B bytes 2/3
   uint32_t VM = 0;
   if (MSK) {
@@ -487,7 +509,7 @@ __device__ __forceinline__ void packed_task(const PackedParams& P, int task, int
   // triple-buffer offsets of the forward-score chunks: row i lives in buffer i % 3, row i+2 in buffer (i+2) % 3 =
   // (i-1) % 3; rotated once per row instead of dividing by 3 (a lane's active rows are consecutive, from 1)
   int fcur_off = kFBuf, fnxt_off = 0;
-  long long cnt[2] = {0, 0};
+  uint32_t cnt[2] = {0u, 0u};  // near-optimal cells of this lane: at most 16 * Lq
   RowSum fin[2] = {{kNeg32, 0, kNeg32, kNeg32}, {kNeg32, 0, kNeg32, kNeg32}};
 
   // What the final cell needs from this lane's 16 columns (RowSum) is M(Lq,.) and F(Lq,Lt).  The loop-carried state
@@ -495,16 +517,21 @@ __device__ __forceinline__ void packed_task(const PackedParams& P, int task, int
   // loop when Lq = 1), and the two halves of a couple get there at different steps.  A rare branch at that point
   // only parks the raw registers in local memory (volatile: the compiler otherwise promotes the arrays to 66 more
   // registers); the summary itself is computed after the loop.  Computing it inside the loop cost ~50 registers.
+  // RB: the lane has stored M(Lq, .) of its 16 columns itself (skew row Lq - 1 + off of the score blob, LOC clamp
+  // included), and F(Lq, Lt) is always register 15 of the segment's last lane in the right-aligned forward pass: one
+  // branch-free select per step keeps it (fcol), and nothing is parked.
   volatile uint32_t capX[2][17], capF[2][16];
   int capQ[2] = {0, 0};
+  uint32_t fcol = 0;
   auto capture = [&](int h, int qa) {
 #pragma unroll
     for (int c = 0; c < 16; ++c) { capX[h][c + 1] = Xp[c]; capF[h][c] = Fn[c]; }
     capX[h][0] = xl_hold;
     capQ[h] = qa;
   };
-  for (int h = 0; h < 2; ++h)
-    if (pid[h] >= 0 && Lq[h] == 1) capture(h, (int)qp[h][0]);
+  if (!RB)
+    for (int h = 0; h < 2; ++h)
+      if (pid[h] >= 0 && Lq[h] == 1) capture(h, (int)qp[h][0]);
 
   for (int s = 0; s < nsteps; ++s) {
     uint32_t xn = __shfl_up_sync(0xffffffffu, x_pub, 1);
@@ -521,20 +548,12 @@ __device__ __forceinline__ void packed_task(const PackedParams& P, int task, int
     if (act0 || act1) {
       // One cp.async group is committed per row.  Query blocks are requested 8 rows ahead and forward
       // scores 2 rows ahead, so only the most recent group(s) may still be in flight.
-      if (i == 1) {
-        cp_async_wait_all();
-        qa_n0 = ld1<SA>(qst[0]);
-        qa_n1 = ld1<SA>(qst[1]);
-      } else if (MSK) cp_async_wait_group<1>();
+      if (MSK) cp_async_wait_group<1>();
       else cp_async_wait_group<4>();
 #if AADP_PROF_AHEAD
-      // The profile words of THIS row were loaded during the previous step (the first row loads them here): the
+      // The profile words of THIS row were loaded during the previous step (the first row: before the loop): the
       // step starts with register operands only.  The residue of the next row comes out of the ring now and its
       // profile row follows as soon as the residue is there -- both loads have a whole step to complete.
-      if (i == 1) {
-        pnA = ld16<SA>(profA_s + qa_n0 * W);
-        pnB = ld16<SA>(profB_s + qa_n1 * W);
-      }
       const uint32_t pwA[4] = {pnA.x, pnA.y, pnA.z, pnA.w};
       const uint32_t pwB[4] = {pnB.x, pnB.y, pnB.z, pnB.w};
       qa_n0 = ld1<SA>(qst[0] + (i & 15));
@@ -676,54 +695,66 @@ __device__ __forceinline__ void packed_task(const PackedParams& P, int task, int
       // byte offsets of this step inside a pair's products fit 32 bits (Lt <= 512, bounded Lq): one 32-bit
       // multiply shared by both halves, then base + offset per store
       const uint32_t snl = (uint32_t)s * (uint32_t)nl;
-      if (act0) {
-        if (TBM) *reinterpret_cast<uint2*>(tbp[0] + (size_t)(snl * 8u)) = make_uint2(tbA[0], tbA[1]);
-        if (FST) {
-          uint8_t* d = reinterpret_cast<uint8_t*>(scp[0]) + (size_t)(snl * 32u);
-          *reinterpret_cast<uint4*>(d) = make_uint4(oA[0], oA[1], oA[2], oA[3]);
-          *reinterpret_cast<uint4*>(d + (size_t)((uint32_t)nl * 16u)) = make_uint4(oA[4], oA[5], oA[6], oA[7]);
-        }
-        if (MSK) {
-          *reinterpret_cast<uint16_t*>(mkp[0] + (size_t)(snl * 2u)) = (uint16_t)(accM & 0xffffu);
-          cnt[0] += __popc(accM & 0xffffu);
-        }
+      // every word and address of the step first, then the stores of both halves, predicated in one place
+      uint8_t* const tba = tbp[0] + (size_t)(snl * 8u);
+      uint8_t* const tbb = tbp[1] + (size_t)(snl * 8u);
+      uint8_t* const sca = reinterpret_cast<uint8_t*>(scp[0]) + (size_t)(snl * 32u);
+      uint8_t* const scb = reinterpret_cast<uint8_t*>(scp[1]) + (size_t)(snl * 32u);
+      const size_t sch = (size_t)((uint32_t)nl * 16u);
+      uint8_t* const mka = mkp[0] + (size_t)(snl * 2u);
+      uint8_t* const mkb = mkp[1] + (size_t)(snl * 2u);
+      if (TBM) {
+        stg8_if(tba, tbA[0], tbA[1], act0);
+        stg8_if(tbb, tbB[0], tbB[1], act1);
       }
-      if (act1) {
-        if (TBM) *reinterpret_cast<uint2*>(tbp[1] + (size_t)(snl * 8u)) = make_uint2(tbB[0], tbB[1]);
-        if (FST) {
-          uint8_t* d = reinterpret_cast<uint8_t*>(scp[1]) + (size_t)(snl * 32u);
-          *reinterpret_cast<uint4*>(d) = make_uint4(oB[0], oB[1], oB[2], oB[3]);
-          *reinterpret_cast<uint4*>(d + (size_t)((uint32_t)nl * 16u)) = make_uint4(oB[4], oB[5], oB[6], oB[7]);
-        }
-        if (MSK) {
-          *reinterpret_cast<uint16_t*>(mkp[1] + (size_t)(snl * 2u)) = (uint16_t)(accM >> 16);
-          cnt[1] += __popc(accM >> 16);
-        }
+      if (FST) {
+        stg16_if(sca, oA[0], oA[1], oA[2], oA[3], act0);
+        stg16_if(sca + sch, oA[4], oA[5], oA[6], oA[7], act0);
+        stg16_if(scb, oB[0], oB[1], oB[2], oB[3], act1);
+        stg16_if(scb + sch, oB[4], oB[5], oB[6], oB[7], act1);
       }
+      if (MSK) {
+        stg2_if(mka, accM, act0);
+        stg2_if(mkb, accM >> 16, act1);
+        cnt[0] += act0 ? __popc(accM & 0xffffu) : 0;
+        cnt[1] += act1 ? __popc(accM >> 16) : 0;
+      }
+      if constexpr (RB) {
+        const uint32_t sel = (i + 1 == Lq[0] ? 0x0000ffffu : 0u) | (i + 1 == Lq[1] ? 0xffff0000u : 0u);
+        fcol = (Fn[15] & sel) | (fcol & ~sel);
+      } else {
 #ifndef AADP_EXP_NOCAP  // (timing experiment only: without the capture the final scores are wrong)
-      if (i + 1 == Lq[0] || i + 1 == Lq[1]) {
-        for (int h = 0; h < 2; ++h)
-          if (i + 1 == Lq[h]) capture(h, h ? qa_n1 : qa_n0);
-      }
+        if (i + 1 == Lq[0] || i + 1 == Lq[1]) {
+          for (int h = 0; h < 2; ++h)
+            if (i + 1 == Lq[h]) capture(h, h ? qa_n1 : qa_n0);
+        }
 #endif
+      }
     }
   }
 
-  // ---- final-row summaries from the parked state: M(Lq,j) = sim(Lq,j) + X(Lq-1,j-1)
+  // ---- final-row summaries: M(Lq,j) = sim(Lq,j) + X(Lq-1,j-1) from the parked state, or read back (RB)
   for (int h = 0; h < 2; ++h) {
     if (pid[h] < 0) continue;
     const int8_t* prow = (h ? profB : profA) + capQ[h] * W + lane * 16;
+    uint32_t mrow[8];  // RB: the stored words of this half, biased M of columns 2w (low) and 2w+1 (high)
+    if (RB) {
+      const int16_t* row = scp[h] + (size_t)(Lq[h] - 1 + off) * (size_t)(nl * 16);
+      const uint4 a = *reinterpret_cast<const uint4*>(row), b = *reinterpret_cast<const uint4*>(row + nl * 8);
+      mrow[0] = a.x; mrow[1] = a.y; mrow[2] = a.z; mrow[3] = a.w;
+      mrow[4] = b.x; mrow[5] = b.y; mrow[6] = b.z; mrow[7] = b.w;
+    }
     RowSum r = {kNeg32, 0, kNeg32, kNeg32};
     for (int c = 0; c < 16; ++c) {
       const int j = off * 16 + c + 1 - sig[h];
-      int m = unb16(capX[h][c], h) + (int)prow[c];  // M(Lq, j)
+      int m = RB ? unb16(mrow[c >> 1], c & 1) : unb16(capX[h][c], h) + (int)prow[c];  // M(Lq, j)
       if (LOC) m = max(m, 0);
       if (j >= 1 && j < Lt[h]) {
         const int v = m - (S.delfree ? 0 : gap_w(gi, ge, Lt[h] - j));
         if (v > r.rb_val) { r.rb_val = v; r.rb_k = j; }
       } else if (j == Lt[h]) {
         r.diag = m;
-        r.col = (Lq[h] >= 2) ? unb16(capF[h][c], h) + (S.insfree ? gi : 0) : kNeg32;
+        r.col = (Lq[h] >= 2) ? unb16(RB ? fcol : capF[h][c], h) + (S.insfree ? gi : 0) : kNeg32;
       }
     }
     fin[h] = r;
@@ -758,7 +789,7 @@ __device__ __forceinline__ void packed_task(const PackedParams& P, int task, int
     }
     if (MSK && P.count) {
       __syncwarp();
-      reinterpret_cast<long long*>(red)[lane] = cnt[h];
+      reinterpret_cast<long long*>(red)[lane] = (long long)cnt[h];
       __syncwarp();
       if (seg_start && pid[h] >= 0) {
         long long t = 0;
@@ -772,7 +803,7 @@ __device__ __forceinline__ void packed_task(const PackedParams& P, int task, int
   }  // rep
 }
 
-template <int TBM, int FST, int MSK, int XM, int LOC = 0, int PRO = 0>
+template <int TBM, int FST, int MSK, int XM, int LOC = 0, int PRO = 0, int RB = 0>
 __global__ void __launch_bounds__(kPackedWarps * 32) __maxnreg__(XM ? 168 : (MSK ? 255 : (TBM ? 224 : 200))) packed_kernel(const PackedParams P) {
   extern __shared__ __align__(16) unsigned char smem[];
   const int A = P.sc.A;
@@ -792,7 +823,7 @@ __global__ void __launch_bounds__(kPackedWarps * 32) __maxnreg__(XM ? 168 : (MSK
     if (lane == 0) item = atomicAdd(P.counter, 1u);
     item = __shfl_sync(0xffffffffu, item, 0);
     if (item >= (unsigned int)P.n_tasks) break;
-    packed_task<TBM, FST, MSK, XM, LOC, PRO>(P, (int)item, prof, red, stage, lane);
+    packed_task<TBM, FST, MSK, XM, LOC, PRO, RB>(P, (int)item, prof, red, stage, lane);
   }
 }
 

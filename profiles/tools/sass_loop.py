@@ -1,6 +1,6 @@
 """Opcode histogram of the hot loop of a kernel from `cuobjdump -sass` output (no GPU needed).
 
-usage: python profiles/tools/sass_loop.py <lib.so> <kernel-name-substring> [--dump]
+usage: python profiles/tools/sass_loop.py <lib.so> <kernel-name-substring> [--dump] [--reuse]
 The hot loop is taken as the innermost backward branch span that holds the most VIMNMX/FMNMX instructions.
 """
 import collections
@@ -35,7 +35,7 @@ def hot_loop(ins, key=None):
     if key is None:  # the packed kernels are recognised by their int16x2 min/max, the others by any min/max
         key = (".S16x2", ".16x2") if any(".S16x2" in s for _, s in ins) else ("VIMNMX", "FMNMX", "VIADDMNMX")
     addr = [a for a, _ in ins]
-    best = None
+    loops = []
     for i, (a, s) in enumerate(ins):
         m = re.search(r"BRA(?:\.\w+)* (?:`\(\.L_x_\d+\)|0x([0-9a-f]+))", s)
         if not m or not m.group(1):
@@ -48,10 +48,47 @@ def hot_loop(ins, key=None):
             continue
         body = ins[j:i + 1]
         n = sum(1 for _, x in body if any(k in x for k in key))
-        # innermost loop that still holds (nearly) all of the min/max instructions
-        if n and (best is None or n > best[0] * 1.5 or (n >= best[0] * 0.6 and len(body) < len(best[1]))):
-            best = (n, body)
-    return best[1] if best else []
+        if n:
+            loops.append((n, body))
+    # the smallest loop that holds at least half of the min/max instructions of the richest one: the row loop, also
+    # where the compiler has peeled a copy of its body into the enclosing task loop
+    top = max((n for n, _ in loops), default=0)
+    best = min((b for n, b in loops if 2 * n >= top), key=len, default=[])
+    return best
+
+
+def regs(tok, width):
+    m = re.match(r"\[?-?R(\d+)", tok)
+    return set(range(int(m.group(1)), int(m.group(1)) + width)) if m and m.group(1) else set()
+
+
+def width(op, tok):
+    if ".64" in tok or "WIDE" in op:
+        return 2
+    if "[" in tok:  # a 32-bit address (shared memory)
+        return 1
+    return 4 if op.endswith(".128") else (2 if op.endswith(".64") else 1)
+
+
+def store_reuse(body):
+    """Global stores / cp.async in the loop one of whose operand registers is written again before the loop's end."""
+    out = []
+    for k, (a, s) in enumerate(body):
+        op = opcode(s)
+        if not (op.startswith("STG") or op.startswith("LDGSTS")):
+            continue
+        ops = [t.strip() for t in s.split(None, 2 if s.startswith("@") else 1)[-1].split(",")]
+        used = set().union(*(regs(t, width(op, t)) for t in ops))
+        for b, t in body[k + 1:]:
+            top = opcode(t)
+            if top.startswith(("ST", "LDGSTS", "BRA", "BSSY", "BSYNC", "DEPBAR", "LDGDEPBAR", "CCTL", "ISETP", "UI", "UL", "UM", "US", "PLOP")):
+                continue
+            dst = t.split(None, 2 if t.startswith("@") else 1)[-1].split(",")[0].strip()
+            hit = regs(dst, width(top, dst)) & used
+            if hit:
+                out.append((a, s, b, t))
+                break
+    return out
 
 
 if __name__ == "__main__":
@@ -64,6 +101,11 @@ if __name__ == "__main__":
         print(f"== {name}: {len(ins)} instr, hot loop {len(body)} instr [{body[0][0]:#x}..{body[-1][0]:#x}]" if body else f"== {name}: no loop")
         for k, v in h.most_common():
             print(f"   {v:5d} {k}")
+        if "--reuse" in sys.argv:
+            r = store_reuse(body)
+            print(f"   stores whose operand registers are rewritten later in the step: {len(r)}")
+            for a, s, b, t in r:
+                print(f"     {a:06x} {s}  <-  {b:06x} {t}")
         if "--dump" in sys.argv:
             for a, s in body:
                 print(f"  {a:06x} {s}")
